@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- batched OCP SQP solves/sec (H=20 quadrotor MPC) on N B200s, one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one batched CUDA_SQP solve of B instances per GPU (BASELINE.json configs[2]:
@@ -20,14 +20,23 @@ iterate x=0 so that all steps do identical work.
 
 `--impl reference` times the oracle alone (rank 0 only).  torch is used for device memory,
 streams, events and torch.distributed -- not for compute.
+
+`--dump-outputs DIR` writes what the last timed step returned (x [B, N], f [B], stats [B, 12], gathered over the
+ranks) as DIR/<name>.npy in float64, so that two builds can be compared output for output on the same seeded inputs.
+
+The bench writes nothing into the source tree (it may be read-only): stage libraries are looked up in, and if
+missing compiled into, a temporary directory (see private_share_dir).
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -58,6 +67,7 @@ def emit(line: dict):
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
+sys.dont_write_bytecode = True     # no __pycache__ in the tree for the modules imported from it
 
 METRIC = "batched OCP SQP solves/sec (H=20)"
 UNIT = "solves/s"
@@ -81,7 +91,12 @@ def parse_args():
     ap.add_argument("--latency-solves", type=int, default=50)
     ap.add_argument("--secondary", default="auto", choices=["auto", "on", "off"],
                     help="bounded pass over BASELINE.json configs[3]/[4] at their stated total sizes (auto: with >= 2 GPUs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write x, f and stats of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 WORKLOADS = {
@@ -214,6 +229,44 @@ class ClockSampler:
 
 
 # ---------------------------------------------------------------------------------------------
+# files: stage libraries and dumped outputs
+# ---------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def private_share_dir():
+    """Problem() needs a writable share directory for its generated stage library.  Unless OCP_B200_SHARE_DIR names
+    one, the bench uses a temporary directory (removed at exit) in which the stage libraries build() left in the
+    package are linked, so that a model built there is not compiled again and the tree is never written to."""
+    if os.environ.get("OCP_B200_SHARE_DIR"):
+        return
+    share = Path(tempfile.mkdtemp(prefix="ocp_b200_bench_"))
+    atexit.register(shutil.rmtree, share, True)
+    (share / "code_gen").mkdir()
+    for so in (ROOT / "optimal_control_problem_b200" / "share" / "code_gen").glob("*.so"):
+        (share / "code_gen" / so.name).symlink_to(so)
+    os.environ["OCP_B200_SHARE_DIR"] = str(share)
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes every array as out_dir/<name>.npy in float64.  The arrays share their leading (instance) axis; when the
+    files would exceed DUMP_LIMIT_BYTES together, each keeps the same fixed, seeded sample of instances."""
+    rows = next(iter(arrays.values())).shape[0]
+    total = sum(8 * a.size for a in arrays.values())
+    room = DUMP_LIMIT_BYTES - 1024 * len(arrays)       # .npy headers are 128 bytes each
+    if total > room:
+        keep = room * rows // total
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        print(f"bench.py: outputs exceed {DUMP_LIMIT_BYTES / 1e6:.0f} MB, kept {keep} of {rows} instances (seed 0)",
+              file=sys.stderr)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", np.ascontiguousarray(a, dtype=np.float64))
+
+
+# ---------------------------------------------------------------------------------------------
 # the B200 arm
 # ---------------------------------------------------------------------------------------------
 def algorithmic_bytes(dims, nnz_pu, stats, ocp, direct=None):
@@ -301,6 +354,7 @@ def b200_arm(args):
     import torch
     import torch.distributed as dist
 
+    private_share_dir()                  # before the package reads OCP_B200_SHARE_DIR
     import optimal_control_problem_b200 as ocp
     from optimal_control_problem_b200.sharding import gather_shards
 
@@ -370,6 +424,11 @@ def b200_arm(args):
         barrier()
         step_ms.append(e0.elapsed_time(e1))
     t_wall1 = time.perf_counter()
+    if args.dump_outputs:                                # what the last timed step returned, before anything else runs
+        outputs = {"x": gathered.get("x", d_x), "f": gather_shards(d_f, world * B), "stats": gathered.get("stats", d_stats)}
+        outputs = {k: v.cpu().numpy() for k, v in outputs.items()}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
     prof = sol.get_profile(reset=True)
     sol.set_profiling(False)
