@@ -91,7 +91,7 @@ def compile_objects(sources: list[str], flags: list[str], objdir: Path, tag: str
     return objs
 
 
-CUDA_SOURCES = ["csrc/ocp_b200.cu", "csrc/direct_smem.cu", "csrc/direct_mixed.cu", "csrc/direct_multi.cu", "csrc/direct_multi_v3.cu", "csrc/direct_multi_v4.cu", "csrc/direct_big.cu", "csrc/direct_compact.cu"]
+CUDA_SOURCES = ["csrc/ocp_b200.cu", "csrc/direct_smem.cu", "csrc/direct_mixed.cu", "csrc/direct_multi.cu", "csrc/direct_big.cu", "csrc/direct_compact.cu"]
 NVCC_FLAGS = [*ARCH, "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-I" + str(INCLUDE), "-I" + str(PKG / "csrc"),
               *os.environ.get("OCP_B200_NVCC_EXTRA", "").split()]
 

@@ -1,5 +1,5 @@
 // admm_compact_kernel.cuh -- the throughput kernel of the batched ADMM QP solve for sm_100a:
-// FOUR (or three) CTAs per SM, 128 threads each.
+// FOUR CTAs per SM, 128 threads each.
 //
 // Same algorithm, same arithmetic order and the same factorisation / solve code (tri_fast.cuh,
 // tri_twisted.cuh) as admm_direct_kernel.cuh -- OSQP set-up + ADMM + SQP update of B independent QPs,
@@ -45,12 +45,13 @@ struct Layout {
   int s_stride, sp_stride, stage_stride;
   // slab
   size_t dinv, lsub, lp, q, l, u, D, E, pval, dx, dy, an, cn, sx, sz, sy, slab_doubles;
-  bool ok, q_smem, lu_smem, scale_smem;
+  bool ok, q_smem, lu_smem;
 };
 
-// flags: bit 0 = q in shared memory, bit 1 = l and u in shared memory, bit 2 = the scaling vectors D, E and the
-// Ruiz by-products in shared memory (otherwise streamed from the slab)
-constexpr int kQInSmem = 1, kLuInSmem = 2, kScaleInSmem = 4;
+// flags: bit 0 = q in shared memory, bit 1 = l and u in shared memory (otherwise streamed from the slab).  The scaling
+// vectors D, E and the Ruiz by-products stay in the slab: in shared memory as well they made the kernel slower (H = 20
+// quadrotor: 9.6 -> 9.9 ms per launch; the 10 KB are worth more as L1).
+constexpr int kQInSmem = 1, kLuInSmem = 2;
 __host__ __device__ inline Layout make_layout(const PatternDev& P, int arena_words, int flags) {
   auto ev = [](size_t v) { return (v + 1) & ~size_t(1); };
   const size_t n = ev(P.n), m = ev(P.m), np = P.tri_np, bs = P.tri_bs, ld = P.tri_ld, nb = P.tri_nb;
@@ -80,27 +81,20 @@ __host__ __device__ inline Layout make_layout(const PatternDev& P, int arena_wor
   L.xp = o; o += ev(np + 2); guard(o, false);
   L.piv = o; o += 64; guard(o, false);
   L.arena = o; o += ev((size_t(arena_words) + 1) / 2); guard(o, false);
-  size_t qs = 0, ls = 0, us = 0, ds = 0, es = 0, cns = 0;
+  size_t qs = 0, ls = 0, us = 0;
   if (flags & kQInSmem) { qs = o; o += n; guard(o, false); }
   if (flags & kLuInSmem) { ls = o; o += m; guard(o, false); us = o; o += m; guard(o, false); }
-  if (flags & kScaleInSmem) { ds = o; o += n; guard(o, false); es = o; o += m; guard(o, false); cns = o; o += n; guard(o, false); }
   L.smem_doubles = o;
   size_t g = 0;
   L.dinv = g; g += nb * bs * ld; guard(g, true); L.lsub = g; g += nb * bs * ld; guard(g, true); L.lp = g; g += ev(np * nb * bs); guard(g, true);
   L.q_smem = (flags & kQInSmem) != 0; L.lu_smem = (flags & kLuInSmem) != 0;
   if (L.q_smem) L.q = qs; else { L.q = g; g += n; guard(g, true); }
   if (L.lu_smem) { L.l = ls; L.u = us; } else { L.l = g; g += m; guard(g, true); L.u = g; g += m; guard(g, true); }
-  L.scale_smem = (flags & kScaleInSmem) != 0;
   L.pval = g; g += ev(P.nnz_p); guard(g, true); L.dx = g; g += n; guard(g, true); L.dy = g; g += m; guard(g, true);
-  if (L.scale_smem) {
-    L.D = ds; L.E = es; L.cn = cns;
-    L.an = L.x + m;   // behind the row scales on x|w: n_e + m_e - m >= n doubles are left there
-  } else {
-    L.D = g; g += n; guard(g, true); L.E = g; g += m; guard(g, true); L.an = g; g += n; guard(g, true); L.cn = g; g += n; guard(g, true);
-  }
+  L.D = g; g += n; guard(g, true); L.E = g; g += m; guard(g, true); L.an = g; g += n; guard(g, true); L.cn = g; g += n; guard(g, true);
   // parking space of a refactorisation: dx, dy and the Ruiz by-products are dead at that point
   L.sx = L.dx; L.sz = L.dy;
-  if (!L.scale_smem && kCanaryDoubles == 0 && 2 * n >= m) L.sy = L.an;   // (an | cn are contiguous without guards)
+  if (kCanaryDoubles == 0 && 2 * n >= m) L.sy = L.an;   // (an | cn are contiguous without guards)
    else { L.sy = g; g += m; guard(g, true); }
   L.slab_doubles = (g + 15) & ~size_t(15);
   return L;
@@ -426,7 +420,7 @@ __device__ inline void tri_solve_twisted_tmem(const PatternDev& P, const Work& W
   OCP_B200_FINE_LAP(clk, OCP_B200_PHASE_SOLVE_BWD);
 }
 
-template <int BS, bool kTile>   // kTile: chain steps of the factorisation in 2 x 2 tiles (thread groups of 64)
+template <int BS>
 __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, const ocp_b200_settings& S, const SolveArgs& A,
                                       Work& W, const Ctx& X, Reducer& R, int inst, QpResult& out, uint32_t tmem) {
   const int tid = threadIdx.x, T = blockDim.x;
@@ -563,7 +557,7 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
   clk.lap(OCP_B200_PHASE_SCALE);
   direct::tri_assemble_program(P, W, rv, sigma);
   clk.lap(OCP_B200_PHASE_KKT_ASSEMBLE);
-  direct::tri_factor_twisted<BS, true, kTile>(P, W);   // scratch: the iteration vectors (nothing lives there yet)
+  direct::tri_factor_twisted<BS, true, true>(P, W);   // scratch: the iteration vectors (nothing lives there yet)
   if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
   clk.lap(OCP_B200_PHASE_FACTOR);
   // ---- cold start ----
@@ -773,7 +767,7 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
         // (inlined a second time on purpose: an out-of-line copy shared with the set-up was measured slower,
         // 9.6 -> 9.8 ms per launch with P and W passed by value, 11.7 ms by reference)
         direct::tri_assemble_program(P, W, rv, sigma);
-        direct::tri_factor_twisted<BS, true, kTile>(P, W);
+        direct::tri_factor_twisted<BS, true, true>(P, W);
         if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
         for (int j = tid; j < n; j += T) W.x[j] = X.sx[j];
         for (int i = tid; i < m; i += T) {
@@ -807,7 +801,7 @@ admm_compact_kernel(const PatternDev P, const CompactIdx C, const ocp_b200_setti
   __shared__ double red_buf[2 * (kThreads / 32) * kRedWidth];
   __shared__ int s_inst;
   __shared__ uint32_t s_tmem;
-  static_assert(kThreads >= 128, "four sweep warps");
+  static_assert(kThreads == 128, "four sweep warps; the tiled chain steps take thread groups of 64");
   if constexpr (BS == 16) {   // Tensor Memory for the sweep blocks: one warp allocates, the same warp frees it at the end
     if (threadIdx.x < 32) {
       asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
@@ -831,7 +825,7 @@ admm_compact_kernel(const PatternDev P, const CompactIdx C, const ocp_b200_setti
   W.ring_bar = nullptr; W.ring_phase = nullptr; W.ring_slots = 0;
   W.Dinv = gl + L.dinv; W.Lsub = gl + L.lsub; W.Lp = gl + L.lp;
   W.q = (L.q_smem ? sm : gl) + L.q; W.l = (L.lu_smem ? sm : gl) + L.l; W.u = (L.lu_smem ? sm : gl) + L.u;
-  W.D = (L.scale_smem ? sm : gl) + L.D; W.E = (L.scale_smem ? sm : gl) + L.E;
+  W.D = gl + L.D; W.E = gl + L.E;
   W.Pval = gl + L.pval; W.dx = gl + L.dx; W.dy = gl + L.dy;
   W.idx = nullptr; W.phase = nullptr;
   uint32_t* ar = reinterpret_cast<uint32_t*>(sm + L.arena);
@@ -839,8 +833,7 @@ admm_compact_kernel(const PatternDev P, const CompactIdx C, const ocp_b200_setti
   if (kCanaryDoubles > 0 && threadIdx.x == 0)
     for (int gi = 0; gi < L.nguard; ++gi)
       for (int c = 0; c < kCanaryDoubles; ++c) ((L.guard_slab[gi] ? gl : sm) + L.guard_off[gi])[c] = canary_value(gi);
-  Ctx X{ar, sm + L.rscale, sm + L.psm, (L.scale_smem ? sm : gl) + L.an, (L.scale_smem ? sm : gl) + L.cn, gl + L.sx, gl + L.sz,
-        gl + L.sy, gl + L.pval};
+  Ctx X{ar, sm + L.rscale, sm + L.psm, gl + L.an, gl + L.cn, gl + L.sx, gl + L.sz, gl + L.sy, gl + L.pval};
   __syncthreads();
   Reducer R{red_buf, 0, (kThreads / 32) * kRedWidth};
   while (true) {
@@ -850,10 +843,7 @@ admm_compact_kernel(const PatternDev P, const CompactIdx C, const ocp_b200_setti
     __syncthreads();
     if (inst >= A.B) break;
     QpResult res;
-#ifndef OCP_B200_NO_TILE
-#define OCP_B200_NO_TILE 0   // 1: chain steps with one dot product at a time (A/B measurements)
-#endif
-    solve_instance<BS, kThreads == 128 && !OCP_B200_NO_TILE>(P, C, S, A, W, X, R, inst, res, tmem);
+    solve_instance<BS>(P, C, S, A, W, X, R, inst, res, tmem);
     write_outputs(P, A, W.x, W.y, R, inst, res);
   }
   if constexpr (BS == 16) {

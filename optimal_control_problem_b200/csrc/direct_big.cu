@@ -1,32 +1,10 @@
-// Instantiation of admm_direct_kernel<PLACE_BIG, 384, 1> (see direct_launch.h).
-#include "admm_direct_kernel.cuh"
-#include "direct_launch.h"
+// Instantiation of admm_direct_kernel<PLACE_BIG, 384, 1> (see direct_instance.h).
+#include "direct_instance.h"
 
 namespace ocpb200 {
 namespace direct {
 
-#ifndef OCP_B200_BIG_THREADS
-#define OCP_B200_BIG_THREADS 384
-#endif
-#define KERNEL admm_direct_kernel<PLACE_BIG, OCP_B200_BIG_THREADS, 1>
-
-cudaError_t kernel_info_big(KernelInfo* out) {
-  cudaFuncAttributes fa{};
-  cudaError_t e = cudaFuncGetAttributes(&fa, KERNEL);
-  if (e == cudaSuccess) { out->static_smem = static_cast<int>(fa.sharedSizeBytes); out->regs = fa.numRegs; out->threads = OCP_B200_BIG_THREADS; }
-  return e;
-}
-cudaError_t set_max_dynamic_smem_big(int bytes) {
-  return cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-}
-cudaError_t occupancy_big(int dyn_smem, int* per_sm) {
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, KERNEL, OCP_B200_BIG_THREADS, dyn_smem);
-}
-cudaError_t launch_big(int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S,
-                      const SolveArgs& A, uint32_t smem_mask) {
-  KERNEL<<<grid, OCP_B200_BIG_THREADS, dyn_smem, st>>>(P, S, A, smem_mask);
-  return cudaGetLastError();
-}
+const EntryPoints kBig = Instance<PLACE_BIG, 384, 1>::entry_points;
 
 }  // namespace direct
 }  // namespace ocpb200

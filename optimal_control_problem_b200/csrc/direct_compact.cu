@@ -1,52 +1,30 @@
-// Instantiations of compact::admm_compact_kernel<BS, threads, CTAs/SM> (admm_compact_kernel.cuh): the throughput
-// plan for OCP-shaped QPs that are small enough for three or four CTAs per SM.
+// Instantiations of compact::admm_compact_kernel<BS, 128, 4> (admm_compact_kernel.cuh): the throughput plan for
+// OCP-shaped QPs that are small enough for four CTAs per SM.
 #include "admm_compact_kernel.cuh"
-#include "direct_launch.h"
-
-#include <type_traits>
+#include "compact_launch.h"
 
 namespace ocpb200 {
 namespace compact {
 
-// two shapes: 128 threads x 4 CTAs/SM and 192 threads x 3 CTAs/SM (variant 0 / 1)
-template <int BS, int V> struct Shape;
-template <int BS> struct Shape<BS, 0> { static constexpr int T = 128, R = 4; };
-template <int BS> struct Shape<BS, 1> { static constexpr int T = 192, R = 3; };
+using KernelFn = void (*)(PatternDev, CompactIdx, ocp_b200_settings, SolveArgs, int);
 
-template <typename F>
-static auto dispatch(int bs, int variant, F f) {
-  if (bs == 16) return variant == 0 ? f(Shape<16, 0>{}, std::integral_constant<int, 16>{}) : f(Shape<16, 1>{}, std::integral_constant<int, 16>{});
-  return variant == 0 ? f(Shape<20, 0>{}, std::integral_constant<int, 20>{}) : f(Shape<20, 1>{}, std::integral_constant<int, 20>{});
+static KernelFn kernel(int bs) {
+  return bs == 16 ? admm_compact_kernel<16, kCtaThreads, kCtasPerSm> : admm_compact_kernel<20, kCtaThreads, kCtasPerSm>;
 }
 
-cudaError_t kernel_info(int bs, int variant, direct::KernelInfo* out) {
-  return dispatch(bs, variant, [&](auto sh, auto b) {
-    using S = decltype(sh);
-    cudaFuncAttributes fa{};
-    cudaError_t e = cudaFuncGetAttributes(&fa, admm_compact_kernel<decltype(b)::value, S::T, S::R>);
-    if (e == cudaSuccess) { out->static_smem = static_cast<int>(fa.sharedSizeBytes); out->regs = fa.numRegs; out->threads = S::T; }
-    return e;
-  });
+cudaError_t kernel_info(int bs, direct::KernelInfo* out) {
+  cudaFuncAttributes fa{};
+  cudaError_t e = cudaFuncGetAttributes(&fa, kernel(bs));
+  if (e == cudaSuccess) { out->static_smem = static_cast<int>(fa.sharedSizeBytes); out->regs = fa.numRegs; out->threads = kCtaThreads; }
+  return e;
 }
-cudaError_t set_max_dynamic_smem(int bs, int variant, int bytes) {
-  return dispatch(bs, variant, [&](auto sh, auto b) {
-    using S = decltype(sh);
-    return cudaFuncSetAttribute(admm_compact_kernel<decltype(b)::value, S::T, S::R>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  });
+cudaError_t set_max_dynamic_smem(int bs, int bytes) {
+  return cudaFuncSetAttribute(kernel(bs), cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
 }
-cudaError_t occupancy(int bs, int variant, int dyn_smem, int* per_sm) {
-  return dispatch(bs, variant, [&](auto sh, auto b) {
-    using S = decltype(sh);
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, admm_compact_kernel<decltype(b)::value, S::T, S::R>, S::T, dyn_smem);
-  });
-}
-cudaError_t launch(int bs, int variant, int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const CompactIdx& C,
-                   const ocp_b200_settings& S_, const SolveArgs& A, int layout_flags) {
-  return dispatch(bs, variant, [&](auto sh, auto b) {
-    using S = decltype(sh);
-    admm_compact_kernel<decltype(b)::value, S::T, S::R><<<grid, S::T, dyn_smem, st>>>(P, C, S_, A, layout_flags);
-    return cudaGetLastError();
-  });
+cudaError_t launch(int bs, int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const CompactIdx& C,
+                   const ocp_b200_settings& S, const SolveArgs& A, int layout_flags) {
+  kernel(bs)<<<grid, kCtaThreads, dyn_smem, st>>>(P, C, S, A, layout_flags);
+  return cudaGetLastError();
 }
 void plan_sizes(const PatternDev& P, int arena_words, int layout_flags, size_t* smem_doubles, size_t* slab_doubles, bool* ok) {
   const Layout L = make_layout(P, arena_words, layout_flags);

@@ -1,35 +1,13 @@
-// Instantiation of admm_direct_kernel<PLACE_MIXED, 768, 1> (see direct_launch.h).  The mixed placement
+// Instantiation of admm_direct_kernel<PLACE_MIXED, 768, 1> (see direct_instance.h).  The mixed placement
 // serves problems whose matrices and index arrays stay in global memory: its parallel phases are bound by
 // dependent global loads, so they want as many threads as the register file allows (centroidal H=50,
 // 148 instances: 376 ms at 256 threads, 297 at 512, 278 at 768, 298 at 1024).
-#include "admm_direct_kernel.cuh"
-#include "direct_launch.h"
+#include "direct_instance.h"
 
 namespace ocpb200 {
 namespace direct {
 
-#ifndef OCP_B200_MIXED_THREADS
-#define OCP_B200_MIXED_THREADS 768
-#endif
-#define KERNEL admm_direct_kernel<PLACE_MIXED, OCP_B200_MIXED_THREADS, 1>
-
-cudaError_t kernel_info_mixed(KernelInfo* out) {
-  cudaFuncAttributes fa{};
-  cudaError_t e = cudaFuncGetAttributes(&fa, KERNEL);
-  if (e == cudaSuccess) { out->static_smem = static_cast<int>(fa.sharedSizeBytes); out->regs = fa.numRegs; out->threads = OCP_B200_MIXED_THREADS; }
-  return e;
-}
-cudaError_t set_max_dynamic_smem_mixed(int bytes) {
-  return cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-}
-cudaError_t occupancy_mixed(int dyn_smem, int* per_sm) {
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, KERNEL, OCP_B200_MIXED_THREADS, dyn_smem);
-}
-cudaError_t launch_mixed(int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S,
-                      const SolveArgs& A, uint32_t smem_mask) {
-  KERNEL<<<grid, OCP_B200_MIXED_THREADS, dyn_smem, st>>>(P, S, A, smem_mask);
-  return cudaGetLastError();
-}
+const EntryPoints kMixed = Instance<PLACE_MIXED, 768, 1>::entry_points;
 
 }  // namespace direct
 }  // namespace ocpb200

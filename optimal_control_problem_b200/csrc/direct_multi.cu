@@ -1,51 +1,11 @@
-// Throughput plan: admm_direct_kernel<PLACE_MULTI, threads, CTAs per SM> (see direct_launch.h).  The
-// variants are compiled in their own translation units (direct_multi_v*.cu); this one holds the default
-// and the per-process choice:  OCP_B200_MULTI_VARIANT = 192x2 (default) | 192x3 | 128x4  (diagnostics --
-// the occupancy the plan gets still depends on the shared memory the problem needs).
-#include <cstdlib>
-#include <cstring>
-
-#include "direct_multi_variant.h"
-
-DIRECT_MULTI_DEFINE(multi_192x2, 192, 2)
+// Instantiation of admm_direct_kernel<PLACE_MULTI, 192, 2> (see direct_instance.h): the throughput plan for the
+// problems the compact kernel cannot take.
+#include "direct_instance.h"
 
 namespace ocpb200 {
 namespace direct {
 
-DIRECT_MULTI_DECLARE(multi_192x3)
-DIRECT_MULTI_DECLARE(multi_128x4)
-
-static int multi_variant() {
-  static const int v = [] {
-    const char* e = std::getenv("OCP_B200_MULTI_VARIANT");
-    if (e && !std::strcmp(e, "192x3")) return 1;
-    if (e && !std::strcmp(e, "128x4")) return 2;
-    return 0;
-  }();
-  return v;
-}
-
-cudaError_t kernel_info_multi(KernelInfo* out) {
-  const int v = multi_variant();
-  return v == 1 ? kernel_info_multi_192x3(out) : (v == 2 ? kernel_info_multi_128x4(out) : kernel_info_multi_192x2(out));
-}
-cudaError_t set_max_dynamic_smem_multi(int bytes) {
-  const int v = multi_variant();
-  return v == 1 ? set_max_dynamic_smem_multi_192x3(bytes)
-                : (v == 2 ? set_max_dynamic_smem_multi_128x4(bytes) : set_max_dynamic_smem_multi_192x2(bytes));
-}
-cudaError_t occupancy_multi(int dyn_smem, int* per_sm) {
-  const int v = multi_variant();
-  return v == 1 ? occupancy_multi_192x3(dyn_smem, per_sm)
-                : (v == 2 ? occupancy_multi_128x4(dyn_smem, per_sm) : occupancy_multi_192x2(dyn_smem, per_sm));
-}
-cudaError_t launch_multi(int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S,
-                         const SolveArgs& A, uint32_t smem_mask) {
-  const int v = multi_variant();
-  return v == 1 ? launch_multi_192x3(grid, dyn_smem, st, P, S, A, smem_mask)
-                : (v == 2 ? launch_multi_128x4(grid, dyn_smem, st, P, S, A, smem_mask)
-                          : launch_multi_192x2(grid, dyn_smem, st, P, S, A, smem_mask));
-}
+const EntryPoints kMulti = Instance<PLACE_MULTI, 192, 2>::entry_points;
 
 }  // namespace direct
 }  // namespace ocpb200

@@ -1,40 +1,11 @@
-// Instantiation of admm_direct_kernel<PLACE_SMEM, 384, 1> (see direct_launch.h).
-#include "admm_direct_kernel.cuh"
-#include "direct_launch.h"
+// Instantiation of admm_direct_kernel<PLACE_SMEM, 384, 1> (see direct_instance.h), the placement -> entry points
+// lookup and the plan helpers.
+#include "direct_instance.h"
 
 namespace ocpb200 {
 namespace direct {
 
-#define KERNEL admm_direct_kernel<PLACE_SMEM, 384, 1>
-
-cudaError_t kernel_info_smem(KernelInfo* out) {
-  cudaFuncAttributes fa{};
-  cudaError_t e = cudaFuncGetAttributes(&fa, KERNEL);
-  if (e == cudaSuccess) { out->static_smem = static_cast<int>(fa.sharedSizeBytes); out->regs = fa.numRegs; out->threads = 384; }
-  return e;
-}
-cudaError_t set_max_dynamic_smem_smem(int bytes) {
-  return cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-}
-cudaError_t occupancy_smem(int dyn_smem, int* per_sm) {
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, KERNEL, 384, dyn_smem);
-}
-cudaError_t launch_smem(int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S,
-                      const SolveArgs& A, uint32_t smem_mask) {
-  KERNEL<<<grid, 384, dyn_smem, st>>>(P, S, A, smem_mask);
-  return cudaGetLastError();
-}
-
-#define DECL(tag)                                                                                              \
-  cudaError_t kernel_info_##tag(KernelInfo* out);                                                              \
-  cudaError_t set_max_dynamic_smem_##tag(int bytes);                                                           \
-  cudaError_t occupancy_##tag(int dyn_smem, int* per_sm);                                                      \
-  cudaError_t launch_##tag(int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S, \
-                           const SolveArgs& A, uint32_t smem_mask);
-DECL(mixed)
-DECL(multi)
-DECL(big)
-#undef DECL
+const EntryPoints kSmem = Instance<PLACE_SMEM, 384, 1>::entry_points;
 
 size_t plan_array_doubles(const PatternDev& P, int id) { return array_doubles(P, id); }
 int plan_array_count() { return AR_COUNT; }
@@ -48,26 +19,13 @@ void plan_mixed_priority(std::vector<int>& order) {
            AR_AVAL, AR_IDX, AR_PVAL, AR_LP, AR_DINV, AR_LSUB, AR_DX, AR_DY};
 }
 
-cudaError_t kernel_info(int place, KernelInfo* out) {
-  return place == PLACE_SMEM ? kernel_info_smem(out)
-                             : (place == PLACE_MULTI ? kernel_info_multi(out) : (place == PLACE_BIG ? kernel_info_big(out) : kernel_info_mixed(out)));
-}
-cudaError_t set_max_dynamic_smem(int place, int bytes) {
-  return place == PLACE_SMEM ? set_max_dynamic_smem_smem(bytes)
-                             : (place == PLACE_MULTI ? set_max_dynamic_smem_multi(bytes)
-                                                     : (place == PLACE_BIG ? set_max_dynamic_smem_big(bytes) : set_max_dynamic_smem_mixed(bytes)));
-}
-cudaError_t occupancy(int place, int dyn_smem, int* per_sm) {
-  return place == PLACE_SMEM ? occupancy_smem(dyn_smem, per_sm)
-                             : (place == PLACE_MULTI ? occupancy_multi(dyn_smem, per_sm)
-                                                     : (place == PLACE_BIG ? occupancy_big(dyn_smem, per_sm) : occupancy_mixed(dyn_smem, per_sm)));
-}
-cudaError_t launch(int place, int grid, int dyn_smem, cudaStream_t st, const PatternDev& P, const ocp_b200_settings& S,
-                   const SolveArgs& A, uint32_t smem_mask) {
-  return place == PLACE_SMEM ? launch_smem(grid, dyn_smem, st, P, S, A, smem_mask)
-                             : (place == PLACE_MULTI ? launch_multi(grid, dyn_smem, st, P, S, A, smem_mask)
-                                                     : (place == PLACE_BIG ? launch_big(grid, dyn_smem, st, P, S, A, smem_mask)
-                                                                           : launch_mixed(grid, dyn_smem, st, P, S, A, smem_mask)));
+const EntryPoints& entry_points(int place) {
+  switch (place) {
+    case PLACE_SMEM: return kSmem;
+    case PLACE_MULTI: return kMulti;
+    case PLACE_BIG: return kBig;
+    default: return kMixed;
+  }
 }
 
 }  // namespace direct

@@ -104,6 +104,12 @@ struct DevBuf {
 
 int pad8(int v) { return (v + 7) & ~7; }
 
+// rows with at least kLongRow entries are handled by four lanes each in the row-wise products, the others by one
+// thread.  Measured (quadrotor, rows of <= 17 entries): one thread per row beats four lanes per row by 7 %.
+constexpr int kLongRow = 64;
+// slots of the block staging ring: the one-CTA/SM slab plan (PLACE_BIG) takes kStageSlots when shared memory allows
+constexpr int kStageSlots = 8, kStageSlotsMin = 4;
+
 }  // namespace
 
 struct LaunchPlan {
@@ -128,7 +134,7 @@ struct ocp_b200_solver {
   DevBuf<uint32_t> d_arena;
   ocpb200::CompactIdx cidx{};
   int compact_ok = 0;
-  int compact_variant = 0, compact_flags = 0;   // shape (128x4 / 192x3) and which streamed vectors moved into shared memory
+  int compact_flags = 0;   // which streamed vectors moved into shared memory
   // stage library
   void* lib = nullptr;
   model_assemble_fn assemble = nullptr;
@@ -220,11 +226,7 @@ int upload_pattern(ocp_b200_solver* s, int num_blocks, const int* block_ptr) {
   // fall back to Jacobi for such partitions
   if (max_bs > 64) return fail(OCP_B200_ERR_UNSUPPORTED, "preconditioner blocks larger than 64 columns are not supported");
   std::vector<int> rows_long, rows_short;
-  // rows with at least `long_row` entries are handled by four lanes each in the row-wise products,
-  // the others by one thread (OCP_B200_LONG_ROW overrides the threshold for experiments)
-  int long_row = 64;   // measured (quadrotor, rows of <= 17 entries): one thread per row beats four lanes per row by 7 %
-  if (const char* e = std::getenv("OCP_B200_LONG_ROW")) long_row = std::max(1, std::atoi(e));
-  for (int i = 0; i < m; ++i) (rowptr[i + 1] - rowptr[i] >= long_row ? rows_long : rows_short).push_back(i);
+  for (int i = 0; i < m; ++i) (rowptr[i + 1] - rowptr[i] >= kLongRow ? rows_long : rows_short).push_back(i);
 
   if (n + 1 > 65535 || m + 1 > 65535 || s->nnz_a > 65535 || s->nnz_p > 65535)
     return fail(OCP_B200_ERR_UNSUPPORTED, "problem too large for 16-bit index structures (n, m, nnz < 65536)");
@@ -417,14 +419,15 @@ int plan_launch(ocp_b200_solver* s) {
         (D::plan_big_in_smem(id) ? big_smem : big_slab) += sz;
       }
     };
-    s->pat.stage_slots = 4;
+    s->pat.stage_slots = kStageSlotsMin;
     measure();
     auto make_plan = [&](int place, LaunchPlan& L) -> int {
       D::KernelInfo kx{};
-      CUDA_TRY(D::kernel_info(place, &kx));
+      const D::EntryPoints& ep = D::entry_points(place);
+      CUDA_TRY(ep.kernel_info(&kx));
       L.place = place;
       L.threads = kx.threads;
-      CUDA_TRY(D::set_max_dynamic_smem(place, max_optin - kx.static_smem));
+      CUDA_TRY(ep.set_max_dynamic_smem(max_optin - kx.static_smem));
       if (place == 2) {
         L.smem_mask = 0;
         L.smem_bytes = static_cast<int>(multi_smem * sizeof(double));
@@ -459,29 +462,25 @@ int plan_launch(ocp_b200_solver* s) {
         L.slab_doubles = (slab + 15) & ~size_t(15);
       }
       int occ = 1;
-      CUDA_TRY(D::occupancy(place, L.smem_bytes, &occ));
-      // OCP_B200_MAX_CTAS_PER_SM caps the residency the occupancy calculator allows (diagnostics)
-      if (const char* cap = std::getenv("OCP_B200_MAX_CTAS_PER_SM")) occ = std::min(occ, std::max(1, std::atoi(cap)));
+      CUDA_TRY(ep.occupancy(L.smem_bytes, &occ));
       L.max_ctas = std::max(1, occ) * s->num_sms;
       return OCP_B200_OK;
     };
     D::KernelInfo ki{}, km{};
-    CUDA_TRY(D::kernel_info(1, &ki));
-    CUDA_TRY(D::kernel_info(2, &km));
+    CUDA_TRY(D::kSmem.kernel_info(&ki));
+    CUDA_TRY(D::kMulti.kernel_info(&km));
     const bool fits_all = all * sizeof(double) + ki.static_smem <= size_t(max_optin);
     const bool fits_multi = (multi_smem * sizeof(double) + km.static_smem + 1024) * 2 <= size_t(228) * 1024;
     D::KernelInfo kb{};
-    CUDA_TRY(D::kernel_info(3, &kb));
+    CUDA_TRY(D::kBig.kernel_info(&kb));
     bool fits_big = big_smem * sizeof(double) + kb.static_smem <= size_t(max_optin);
     const bool forced_big = env && !std::strcmp(env, "big");
     if (fits_big && ((!fits_all && !fits_multi) || forced_big)) {
       // the 1-CTA/SM slab plan is the only one: widen the staging area to a ring of 4 blocks per
       // sweep chain (asynchronous bulk copies, tri_twisted.cuh) when shared memory allows
-      int want = 8;
-      if (const char* e = std::getenv("OCP_B200_STAGE_SLOTS")) want = std::max(4, std::min(16, std::atoi(e)));
-      s->pat.stage_slots = want;
+      s->pat.stage_slots = kStageSlots;
       measure();
-      if (big_smem * sizeof(double) + kb.static_smem > size_t(max_optin)) { s->pat.stage_slots = 4; measure(); }
+      if (big_smem * sizeof(double) + kb.static_smem > size_t(max_optin)) { s->pat.stage_slots = kStageSlotsMin; measure(); }
     }
     int deep = fits_all ? 1 : (fits_big ? 3 : 0), wide = fits_multi ? 2 : deep;
     if (env && !std::strcmp(env, "multi") && fits_multi) deep = wide = 2;
@@ -490,28 +489,19 @@ int plan_launch(ocp_b200_solver* s) {
     else if (env && !std::strcmp(env, "big") && fits_big) deep = wide = 3;
     RC_TRY(make_plan(deep, s->deep));
     RC_TRY(make_plan(wide, s->wide));
-    // compact throughput plan (admm_compact_kernel.cuh): index templates, streamed slab vectors, three or four
-    // CTAs per SM -- taken when it keeps more threads resident than the plan above (OCP_B200_PLAN=compact forces it,
-    // any other value of OCP_B200_PLAN keeps it out).  OCP_B200_COMPACT_VARIANT = 128x4 | 192x3 picks the shape;
-    // q, then l and u, move from the slab into shared memory while the residency target still holds.
-    s->compact_variant = 0; s->compact_flags = 0;
+    // compact throughput plan (admm_compact_kernel.cuh): index templates, streamed slab vectors, four CTAs per SM --
+    // taken when it keeps more threads resident than the plan above (OCP_B200_PLAN=compact forces it, any other value
+    // of OCP_B200_PLAN keeps it out).  q, then l and u, move from the slab into shared memory while the residency
+    // target still holds.
+    s->compact_flags = 0;
     if (s->compact_ok && (P.tri_bs == 16 || P.tri_bs == 20) && P.tri_ld == P.tri_bs + 2 && (!env || !std::strcmp(env, "compact"))) {
       namespace K = ocpb200::compact;
-      // measured on the H = 20 quadrotor: 9.6 ms per launch for both shapes with the sweep blocks in the L2 slab; with
-      // them in Tensor Memory 128x4 (8.55 ms) is ahead of 192x3 (8.84 ms)
-      int variant = 0;
-      if (const char* e = std::getenv("OCP_B200_COMPACT_VARIANT")) variant = !std::strcmp(e, "192x3") ? 1 : 0;
-      const int target = variant == 0 ? 4 : 3;
       D::KernelInfo kc{};
-      CUDA_TRY(K::kernel_info(P.tri_bs, variant, &kc));
-      CUDA_TRY(K::set_max_dynamic_smem(P.tri_bs, variant, max_optin - kc.static_smem));
+      CUDA_TRY(K::kernel_info(P.tri_bs, &kc));
+      CUDA_TRY(K::set_max_dynamic_smem(P.tri_bs, max_optin - kc.static_smem));
       int best_flags = -1, best_occ = 0;
       size_t best_sm = 0, best_sl = 0;
-      // (kScaleInSmem -- D, E and the Ruiz by-products in shared memory as well -- was measured: 9.6 -> 9.9 ms per
-      //  launch on the H = 20 quadrotor, the 10 KB are worth more as L1; OCP_B200_COMPACT_FLAGS=7 selects it)
-      std::vector<int> flag_list{3, 1, 0};
-      if (const char* e = std::getenv("OCP_B200_COMPACT_FLAGS")) flag_list = {std::atoi(e) & 7};
-      for (int flags : flag_list) {   // most shared memory first
+      for (int flags : {3, 1, 0}) {   // most shared memory first
         size_t sm_d = 0, sl_d = 0;
         bool lay_ok = false;
         K::plan_sizes(P, s->cidx.arena_words, flags, &sm_d, &sl_d, &lay_ok);
@@ -528,16 +518,14 @@ int plan_launch(ocp_b200_solver* s) {
           occ = std::min({regs_sm / std::max(1, regs_cta), static_cast<int>(size_t(smem_sm) / smem_cta), 2048 / kc.threads,
                           P.tri_bs == 16 ? 512 / 128 : 32});
         }
-        if (occ > best_occ && best_occ < target) { best_occ = occ; best_flags = flags; best_sm = sm_d; best_sl = sl_d; }
+        if (occ > best_occ && best_occ < K::kCtasPerSm) { best_occ = occ; best_flags = flags; best_sm = sm_d; best_sl = sl_d; }
       }
       if (best_flags >= 0) {
-        int occ = std::min(best_occ, target);
-        if (const char* f = std::getenv("OCP_B200_FORCE_CTAS_PER_SM")) occ = std::max(1, std::atoi(f));   // experiment: ignore the occupancy calculator
-        if (const char* cap = std::getenv("OCP_B200_MAX_CTAS_PER_SM")) occ = std::min(occ, std::max(1, std::atoi(cap)));
+        const int occ = std::min(best_occ, K::kCtasPerSm);
         if (occ * kc.threads > (s->wide.max_ctas / s->num_sms) * s->wide.threads || env) {
           s->wide.place = 4; s->wide.threads = kc.threads; s->wide.smem_bytes = static_cast<int>(best_sm * sizeof(double));
           s->wide.smem_mask = 0; s->wide.slab_doubles = best_sl; s->wide.max_ctas = occ * s->num_sms;
-          s->compact_variant = variant; s->compact_flags = best_flags;
+          s->compact_flags = best_flags;
           if (env) s->deep = s->wide;
         }
       }
@@ -654,9 +642,9 @@ int launch_admm(ocp_b200_solver* s, SolveArgs& A, cudaStream_t st) {
       A.slab = s->slab.p;
     }
     if (L.place == 4)
-      CUDA_TRY(ocpb200::compact::launch(s->pat.tri_bs, s->compact_variant, grid, L.smem_bytes, st, s->pat, s->cidx, s->settings, A, s->compact_flags));
+      CUDA_TRY(ocpb200::compact::launch(s->pat.tri_bs, grid, L.smem_bytes, st, s->pat, s->cidx, s->settings, A, s->compact_flags));
     else
-      CUDA_TRY(ocpb200::direct::launch(L.place, grid, L.smem_bytes, st, s->pat, s->settings, A, L.smem_mask));
+      CUDA_TRY(ocpb200::direct::entry_points(L.place).launch(grid, L.smem_bytes, st, s->pat, s->settings, A, L.smem_mask));
   } else if (s->resident) {
     A.slab = nullptr; A.slab_doubles = 0;
     ocp_b200_settings t = s->settings;

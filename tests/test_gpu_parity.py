@@ -471,6 +471,7 @@ def test_iteration_limit_statuses(problems, native, max_iter, eps):
     ("cartpole", 27, "mixed"),
     ("centroidal", 6, "mixed"),    # blocks of 36 (compile-time streamed code), border of 24: wide-border path
     ("cartpole", 40, "big"),       # blocks of 20, twisted sweeps through the two-chain ring
+    ("quadrotor", 5, "multi"),     # two CTAs per SM, factor blocks in the slab
 ])
 def test_streamed_factor_paths_match_oracle(native, monkeypatch, name, horizon, plan):
     """The slab-resident (streamed) factor code on problems small enough to compare quickly: the launch

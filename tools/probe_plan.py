@@ -1,6 +1,6 @@
-"""ADMM kernel time and per-phase SM cycles (CTA 0) of one launch plan at a given residency cap.
-  python tools/probe_plan.py <plan: compact|multi|smem> <cap> [problem] [horizon] [batch]
-Prints one JSON line.  (The plan and the cap are read from the environment when the handle is created.)"""
+"""ADMM kernel time and per-phase SM cycles (CTA 0) of one launch plan.
+  python tools/probe_plan.py <plan: compact|multi|smem> [problem] [horizon] [batch]
+Prints one JSON line.  (The plan is read from the environment when the handle is created.)"""
 import json
 import os
 import sys
@@ -8,12 +8,11 @@ from pathlib import Path
 
 import numpy as np
 
-plan, cap = sys.argv[1], sys.argv[2]
-name = sys.argv[3] if len(sys.argv) > 3 else "quadrotor"
-horizon = int(sys.argv[4]) if len(sys.argv) > 4 else 0
-B = int(sys.argv[5]) if len(sys.argv) > 5 else 4096
+plan = sys.argv[1]
+name = sys.argv[2] if len(sys.argv) > 2 else "quadrotor"
+horizon = int(sys.argv[3]) if len(sys.argv) > 3 else 0
+B = int(sys.argv[4]) if len(sys.argv) > 4 else 4096
 os.environ["OCP_B200_PLAN"] = plan
-os.environ["OCP_B200_MAX_CTAS_PER_SM"] = cap
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import optimal_control_problem_b200 as ocp  # noqa: E402
 
@@ -27,7 +26,7 @@ for _ in range(2):
     x[:] = 0
     sol.solve_batch(frames, refs, prob.lbx, prob.ubx, prob.lbg, prob.ubg, x, None, st)
 prof = sol.get_profile()
-out = {"plan": plan, "cap": cap, "problem": name, "B": B, "wide": sol.launch_plan()["wide"],
+out = {"plan": plan, "problem": name, "B": B, "wide": sol.launch_plan()["wide"],
        "admm_ms_per_launch": round(prof["admm"]["ms"] / prof["admm"]["launches"], 4)}
 # phase cycles: one instance per CTA, every SM at its residency
 per_sm = out["wide"]["ctas_per_sm"]

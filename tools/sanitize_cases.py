@@ -1,7 +1,7 @@
 """Small solves through every placement of the ADMM kernels, for compute-sanitizer (one tool per gpurun call):
   compute-sanitizer --tool memcheck  python tools/sanitize_cases.py
   compute-sanitizer --tool racecheck python tools/sanitize_cases.py
-Placements: all-shared (deep), two-CTA multi, compact (192x3 and 128x4), big (two-chain bulk-copy ring), mixed (streamed
+Placements: all-shared (deep), two-CTA multi, compact, big (two-chain bulk-copy ring), mixed (streamed
 generic blocks), PCG fallback; plus the assembly, objective and shift kernels that every solve launches.  Each case is
 checked against the oracle so that a "clean" run is also a correct one."""
 import os
@@ -18,12 +18,11 @@ import optimal_control_problem_b200 as ocp  # noqa: E402
 CASES = [  # (label, problem, horizon, env)
     ("smem (deep plan)", "quadrotor", 5, {"OCP_B200_PLAN": "smem"}),
     ("multi 192x2", "quadrotor", 5, {"OCP_B200_PLAN": "multi"}),
-    ("compact 192x3", "quadrotor", 5, {"OCP_B200_PLAN": "compact", "OCP_B200_COMPACT_VARIANT": "192x3"}),
-    ("compact 128x4", "quadrotor", 5, {"OCP_B200_PLAN": "compact", "OCP_B200_COMPACT_VARIANT": "128x4"}),
+    ("compact", "quadrotor", 5, {"OCP_B200_PLAN": "compact"}),
     ("big (twisted ring)", "cartpole", 16, {"OCP_B200_PLAN": "big", "OCP_B200_FORCE_STREAM": "1"}),
     ("mixed (streamed blocks)", "centroidal", 3, {"OCP_B200_PLAN": "mixed", "OCP_B200_FORCE_STREAM": "1"}),
 ]
-KEYS = ("OCP_B200_PLAN", "OCP_B200_FORCE_STREAM", "OCP_B200_COMPACT_VARIANT")
+KEYS = ("OCP_B200_PLAN", "OCP_B200_FORCE_STREAM")
 
 ok = True
 for label, name, H, env in CASES:
