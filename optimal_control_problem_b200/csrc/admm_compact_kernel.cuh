@@ -372,11 +372,13 @@ __device__ inline void tri_solve_twisted_tmem(const PatternDev& P, const Work& W
         double v = 0.0;
         if (j < N) {
           {
-            const double2* d2 = reinterpret_cast<const double2*>(W.Dinv + size_t(k) * BS * ld + r1 * ld);
+            // D_k^-1 is stored column-major (tri_factor_twisted<.., kInvT>): the row of thread (k, r1) is a stride-BS
+            // gather, and the 16 threads of a block read 128 contiguous bytes per element
+            const double* dk = W.Dinv + size_t(k) * BS * ld + r1;
             const double* yk = bx + k * BS;
             double dr[BS];
 #pragma unroll
-            for (int t = 0; t < BS / 2; ++t) { const double2 x = d2[t]; dr[2 * t] = x.x; dr[2 * t + 1] = x.y; }
+            for (int t = 0; t < BS; ++t) dr[t] = dk[t * BS];
             double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
 #pragma unroll
             for (int t = 0; t < BS; t += 4) {
@@ -557,7 +559,7 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
   clk.lap(OCP_B200_PHASE_SCALE);
   direct::tri_assemble_program(P, W, rv, sigma);
   clk.lap(OCP_B200_PHASE_KKT_ASSEMBLE);
-  direct::tri_factor_twisted<BS, true, true>(P, W);   // scratch: the iteration vectors (nothing lives there yet)
+  direct::tri_factor_twisted<BS, true, true, BS == 16>(P, W);   // scratch: the iteration vectors (nothing lives there yet)
   if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
   clk.lap(OCP_B200_PHASE_FACTOR);
   // ---- cold start ----
@@ -767,7 +769,7 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
         // (inlined a second time on purpose: an out-of-line copy shared with the set-up was measured slower,
         // 9.6 -> 9.8 ms per launch with P and W passed by value, 11.7 ms by reference)
         direct::tri_assemble_program(P, W, rv, sigma);
-        direct::tri_factor_twisted<BS, true, true>(P, W);
+        direct::tri_factor_twisted<BS, true, true, BS == 16>(P, W);
         if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
         for (int j = tid; j < n; j += T) W.x[j] = X.sx[j];
         for (int i = tid; i < m; i += T) {

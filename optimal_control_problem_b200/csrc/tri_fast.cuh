@@ -112,7 +112,9 @@ __device__ __forceinline__ void tile_cs(const double* __restrict__ a0, const dou
 // lane k broadcasts 1 / M[k][k] (one shuffle), every lane forms its own f[r] with one multiply and
 // the 16 values are all-gathered through `piv` (16-byte aligned scratch of >= BS doubles).  The
 // serial part of a pivot is reciprocal -> shuffle -> multiply -> store/load round trip -> FMAs.
-template <int BS, int LD = BS + 2>
+// kStoreT: the inverse is stored column-major with pitch BS (element (r, c) at M[c * BS + r]) in the first BS * BS
+// doubles of the block; the input is read row-major with pitch LD as always.
+template <int BS, int LD = BS + 2, bool kStoreT = false>
 __device__ __forceinline__ void warp_invert_exact(double* M, int /*ld*/, int lane, double* piv) {
   constexpr int ld = LD;
   static_assert(BS % 2 == 0 && BS <= 32, "one column per lane, even size");
@@ -148,8 +150,14 @@ __device__ __forceinline__ void warp_invert_exact(double* M, int /*ld*/, int lan
     __syncwarp();
   }
   if (act) {
+    if constexpr (kStoreT) {   // (every lane read its column before the first __syncwarp above: in place is safe)
+      double2* out = reinterpret_cast<double2*>(M + lane * BS);
 #pragma unroll
-    for (int r = 0; r < BS; ++r) M[r * ld + lane] = col[r];
+      for (int r = 0; r < BS / 2; ++r) out[r] = make_double2(col[2 * r], col[2 * r + 1]);
+    } else {
+#pragma unroll
+      for (int r = 0; r < BS; ++r) M[r * ld + lane] = col[r];
+    }
   }
 }
 

@@ -30,7 +30,9 @@ __device__ __forceinline__ void group_barrier(int id, int nthreads) {
 // load with LDS instead of generic loads.
 // kTile: the dot products as 2 x 2 tiles (tri_fast.cuh: same bits, a third of the shared-memory loads) -- for thread
 // groups of at most BS * BS / 4 threads, where every thread has at least four results per loop anyway.
-template <int BS, bool kTop, bool kStaged = false, bool kTile = false>
+// kInvT: the inverted blocks D_pred^-1 are stored column-major with pitch BS (warp_invert_exact<.., true>); the staging
+// copy transposes D_pred^-1 back to the row layout the dot products read.
+template <int BS, bool kTop, bool kStaged = false, bool kTile = false, bool kInvT = false>
 __device__ __forceinline__ void chain_step(const Work& W, int np, int N, int /*ld*/, int k, int pred, int slot, double* S,
                                            double* Sp, double* Dpacc, int gt, int GT, int bar, double* stage, double* F = nullptr) {
   constexpr int bb = BS * BS, ld = BS + 2;   // compile-time pitch: addresses fold into immediates
@@ -42,12 +44,19 @@ __device__ __forceinline__ void chain_step(const Work& W, int np, int N, int /*l
   // copy the two blocks this step multiplies into shared memory once (coalesced 16-byte loads).
   const double* C = Cg;
   const double* Dm = Dg;
+  static_assert(!kInvT || kStaged, "a column-major D^-1 is read through the staging copy");
   if (kStaged || stage != nullptr) {
     double2* cs = reinterpret_cast<double2*>(stage);
     double2* ds = reinterpret_cast<double2*>(stage + W.stage_stride);
     const double2* cg2 = reinterpret_cast<const double2*>(Cg);
     const double2* dg2 = reinterpret_cast<const double2*>(Dg);
-    for (int e = gt; e < BS * ld / 2; e += GT) { cs[e] = cg2[e]; ds[e] = dg2[e]; }
+    if constexpr (kInvT) {
+      for (int e = gt; e < BS * ld / 2; e += GT) cs[e] = cg2[e];
+      double* dd = stage + W.stage_stride;
+      for (int e = gt; e < bb; e += GT) dd[(e % BS) * ld + e / BS] = Dg[e];
+    } else {
+      for (int e = gt; e < BS * ld / 2; e += GT) { cs[e] = cg2[e]; ds[e] = dg2[e]; }
+    }
     group_barrier(bar, GT);
     C = stage; Dm = stage + W.stage_stride;
   }
@@ -142,7 +151,7 @@ __device__ __forceinline__ void chain_step(const Work& W, int np, int N, int /*l
   group_barrier(bar, GT);
 }
 
-template <int BS, bool kStaged = false, bool kTile = false>
+template <int BS, bool kStaged = false, bool kTile = false, bool kInvT = false>
 __device__ inline void tri_factor_twisted(const PatternDev& P, const Work& W) {
   const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31;
   const int np = P.tri_np, nb = P.tri_nb, N = nb * BS;
@@ -161,27 +170,27 @@ __device__ inline void tri_factor_twisted(const PatternDev& P, const Work& W) {
   if (grp == 0) {
     OCP_B200_FINE_CLOCK(clk, W.phase);
     for (int k = 0; k < mid; ++k) {           // blocks 0..mid-1; step into k+1 (the last one is mid)
-      if (gt < 32) warp_invert_exact<BS>(W.Dinv + size_t(k) * BS * ld, ld, lane, piv);
+      if (gt < 32) warp_invert_exact<BS, BS + 2, kInvT>(W.Dinv + size_t(k) * BS * ld, ld, lane, piv);
       group_barrier(1, GT);
       OCP_B200_FINE_LAP(clk, OCP_B200_PHASE_FACTOR_INVERT);
-      chain_step<BS, true, kStaged, kTile>(W, np, N, ld, k + 1, k, k + 1, S, Sp, Dpacc, gt, GT, 1, stage, F);
+      chain_step<BS, true, kStaged, kTile, kInvT>(W, np, N, ld, k + 1, k, k + 1, S, Sp, Dpacc, gt, GT, 1, stage, F);
       OCP_B200_FINE_LAP(clk, OCP_B200_PHASE_FACTOR_STEP);
     }
   } else {
     for (int k = nb - 1; k > mid + 1; --k) {  // blocks nb-1..mid+2; step into k-1 (>= mid+1)
-      if (gt < 32) warp_invert_exact<BS>(W.Dinv + size_t(k) * BS * ld, ld, lane, piv);
+      if (gt < 32) warp_invert_exact<BS, BS + 2, kInvT>(W.Dinv + size_t(k) * BS * ld, ld, lane, piv);
       group_barrier(2, GT);
-      chain_step<BS, false, kStaged, kTile>(W, np, N, ld, k - 1, k, k, S, Sp, Dpacc, gt, GT, 2, stage, F);
+      chain_step<BS, false, kStaged, kTile, kInvT>(W, np, N, ld, k - 1, k, k, S, Sp, Dpacc, gt, GT, 2, stage, F);
     }
     if (mid + 1 < nb) {                       // block mid+1: inverted here, eliminated into mid below
-      if (gt < 32) warp_invert_exact<BS>(W.Dinv + size_t(mid + 1) * BS * ld, ld, lane, piv);
+      if (gt < 32) warp_invert_exact<BS, BS + 2, kInvT>(W.Dinv + size_t(mid + 1) * BS * ld, ld, lane, piv);
       group_barrier(2, GT);
     }
   }
   __syncthreads();
   // the bottom chain's last step lands on block mid as well: run it with the whole CTA
-  if (mid + 1 < nb) chain_step<BS, false, kStaged, kTile>(W, np, N, ld, mid, mid + 1, mid + 1, W.S, W.Sp, W.Dp2, tid, T, 0, W.stage, W.Fb);
-  if (tid < 32) warp_invert_exact<BS>(W.Dinv + size_t(mid) * BS * ld, ld, lane, W.piv);
+  if (mid + 1 < nb) chain_step<BS, false, kStaged, kTile, kInvT>(W, np, N, ld, mid, mid + 1, mid + 1, W.S, W.Sp, W.Dp2, tid, T, 0, W.stage, W.Fb);
+  if (tid < 32) warp_invert_exact<BS, BS + 2, kInvT>(W.Dinv + size_t(mid) * BS * ld, ld, lane, W.piv);
   __syncthreads();
   // border of the last block, then D_p = K_pp - (accumulated) - V_mid L_p,mid', inverted
   if (np > 0) {
@@ -194,7 +203,7 @@ __device__ inline void tri_factor_twisted(const PatternDev& P, const Work& W) {
     __syncthreads();
     for (int e = tid; e < pb; e += T) {
       const int r = e / BS, c = e % BS;
-      const double f = dot_cc<BS>(W.Sp + r * BS, Dm + c * ld);
+      const double f = kInvT ? dot_cs<BS>(W.Sp + r * BS, Dm + c, BS) : dot_cc<BS>(W.Sp + r * BS, Dm + c * ld);
       W.Lp[size_t(r) * N + mid * BS + c] = f;
       if (kStaged || W.Fb != nullptr) W.Fb[e] = f;
     }
