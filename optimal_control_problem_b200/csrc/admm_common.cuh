@@ -1,6 +1,8 @@
-// admm_common.cuh -- pieces shared by the two batched ADMM QP kernels for sm_100a
+// admm_common.cuh -- pieces shared by the batched ADMM QP kernels for sm_100a
 // (admm_direct_kernel.cuh: bordered block-tridiagonal LDL' of the reduced KKT matrix;
-//  admm_pcg_kernel.cuh: preconditioned CG on the same matrix for patterns without that structure).
+//  admm_compact_kernel.cuh: the same solve with the per-instance state packed for four CTAs per SM;
+//  admm_pcg_kernel.cuh: preconditioned CG on the same matrix for patterns without that structure),
+// among them the whole OSQP decision layer (update_info, check_termination, adapt_rho, store_solution).
 #pragma once
 
 #include <cuda_runtime.h>
@@ -191,6 +193,16 @@ __device__ __forceinline__ double col_dot_P(const PatternDev& P, const double* _
   return s;
 }
 
+// The sparse products of the OSQP layer below over the CSC / CSR arrays of PatternDev (direct and PCG kernels;
+// the compact kernel has its own over the stage-periodic templates).
+struct PatternOps {
+  const PatternDev& P;
+  template <typename F>
+  __device__ __forceinline__ void for_rows_A(const double* Aval, const double* src, F f) const { ocpb200::for_rows_A(P, Aval, src, f); }
+  __device__ __forceinline__ double col_dot_A(const double* Aval, const double* v, int j) const { return ocpb200::col_dot_A(P, Aval, v, j); }
+  __device__ __forceinline__ double col_dot_P(const double* Pval, const double* v, int j) const { return ocpb200::col_dot_P(P, Pval, v, j); }
+};
+
 // cycle accounting of CTA 0 (diagnostics; see ocp_b200_get_phase_cycles)
 struct PhaseClock {
   long long* out; long long t0;
@@ -259,6 +271,217 @@ __device__ inline void write_outputs(const PatternDev& P, const SolveArgs& A, co
       s[OCP_B200_STAT_STEP_NORM] = sqrt(nrm[0]);
     }
   }
+  __syncthreads();
+}
+
+// ---------------------------------------------------------------------------------------
+// The OSQP decision layer of the three kernels: residuals, termination and infeasibility
+// certificates, rho adaptation, trace and solution store.  The sparse products go through
+// Ops (PatternOps, or compact::CompactOps), which supplies col_dot_A, col_dot_P and
+// for_rows_A; each kernel keeps its own row product and reduction order.
+// ---------------------------------------------------------------------------------------
+
+// persistent kernels: the CTA pulls its next instance from A.counter (done at A.B);
+// s_inst: one int of shared memory
+__device__ __forceinline__ int next_instance(const SolveArgs& A, int& s_inst) {
+  if (threadIdx.x == 0) s_inst = atomicAdd(A.counter, 1);
+  __syncthreads();
+  const int inst = s_inst;
+  __syncthreads();
+  return inst;
+}
+
+// set_rho_vec: -1 free (both bounds infinite), 1 equality, 0 inequality, from the scaled bounds
+__device__ __forceinline__ signed char constraint_type(double lo, double hi) {
+  if (lo < -kInfty * kMinScaling && hi > kInfty * kMinScaling) return -1;
+  return hi - lo < kRhoTol ? 1 : 0;
+}
+
+// OSQP without wall-clock profiling: 4 x check_termination, or ADAPTIVE_RHO_FIXED = 100 iterations when checks are off
+__device__ __forceinline__ int rho_interval(const ocp_b200_settings& S) {
+  return S.adaptive_rho_interval > 0 ? S.adaptive_rho_interval : (S.check_termination > 0 ? 4 * S.check_termination : 100);
+}
+
+// what ADMM iteration iter (1-based) does after its update: residuals are needed for any of the three
+struct IterFlags {
+  bool can_check, last_iter, rho_time;
+  __device__ __forceinline__ IterFlags(const ocp_b200_settings& S, int interval, int iter)
+      : can_check(S.check_termination > 0 && (iter % S.check_termination == 0)),
+        last_iter(iter == S.admm_max_iter),
+        rho_time(S.adaptive_rho && interval > 0 && (iter % interval == 0)) {}
+  __device__ __forceinline__ bool want_info() const { return can_check || rho_time || last_iter; }
+};
+
+// The per-instance vectors of the scaled problem the decision layer reads, wherever the kernel keeps them
+// (shared memory or slab).  dx, dy: the last ADMM step; is_primal_infeasible projects dy in place,
+// store_solution unscales x and y in place.
+struct QpVec {
+  int n, m;
+  const double *Aval, *Pval, *q, *l, *u, *D, *E, *z;
+  double *x, *y, *dx, *dy;
+};
+// (built where it is used: pointers held across the iteration loop cost registers in every phase, DESIGN.md 5.5)
+template <class Work>
+__device__ __forceinline__ QpVec qp_vectors(const Work& W, int n, int m) {
+  return QpVec{n, m, W.Aval, W.Pval, W.q, W.l, W.u, W.D, W.E, W.z, W.x, W.y, W.dx, W.dy};
+}
+
+// update_info: the inf-norms behind the residuals and their tolerances, unscaled (U) and scaled (S).
+// Kept as one array so that one block reduction of kRedWidth values serves them all.
+enum InfoSlot {
+  kPrimU, kAxU, kZU,          // E^-1 (Ax - z), E^-1 Ax, E^-1 z
+  kPrimS, kAxS, kZS,          //      Ax - z,        Ax,       z
+  kDualU, kQU, kPxU, kAtyU,   // D^-1 (q + Px + A'y), D^-1 q, D^-1 Px, D^-1 A'y  (times 1/c when used)
+  kDualS, kQS, kPxS, kAtyS,   //      q + Px + A'y,        q,      Px,      A'y
+  kNumInfo
+};
+static_assert(kNumInfo <= kRedWidth, "the residual norms are reduced in one call");
+
+template <class Ops>
+__device__ __forceinline__ void update_info(const Ops& I, const QpVec& V, Reducer& R, double (&mx)[kRedWidth]) {
+#pragma unroll
+  for (int k = 0; k < kRedWidth; ++k) mx[k] = 0.0;
+  I.for_rows_A(V.Aval, V.x, [&](int i, double ax) {
+    const double einv = 1.0 / V.E[i];
+    const double zi = V.z[i];
+    const double rp = ax - zi;
+    mx[kPrimU] = fmax(mx[kPrimU], fabs(einv * rp));
+    mx[kAxU] = fmax(mx[kAxU], fabs(einv * ax));
+    mx[kZU] = fmax(mx[kZU], fabs(einv * zi));
+    mx[kPrimS] = fmax(mx[kPrimS], fabs(rp));
+    mx[kAxS] = fmax(mx[kAxS], fabs(ax));
+    mx[kZS] = fmax(mx[kZS], fabs(zi));
+  });
+  for (int j = threadIdx.x; j < V.n; j += blockDim.x) {
+    const double dinv = 1.0 / V.D[j];
+    const double qj = V.q[j];
+    const double px = I.col_dot_P(V.Pval, V.x, j);
+    const double aty = I.col_dot_A(V.Aval, V.y, j);
+    const double rd = qj + px + aty;
+    mx[kDualU] = fmax(mx[kDualU], fabs(dinv * rd));
+    mx[kQU] = fmax(mx[kQU], fabs(dinv * qj));
+    mx[kPxU] = fmax(mx[kPxU], fabs(dinv * px));
+    mx[kAtyU] = fmax(mx[kAtyU], fabs(dinv * aty));
+    mx[kDualS] = fmax(mx[kDualS], fabs(rd));
+    mx[kQS] = fmax(mx[kQS], fabs(qj));
+    mx[kPxS] = fmax(mx[kPxS], fabs(px));
+    mx[kAtyS] = fmax(mx[kAtyS], fabs(aty));
+  }
+  block_reduce<kRedWidth, true>(mx, R);
+}
+
+// residuals of the unscaled problem (c: cost scaling of the Ruiz equilibration, cinv = 1 / c)
+__device__ __forceinline__ double prim_residual(const double (&mx)[kRedWidth]) { return mx[kPrimU]; }
+__device__ __forceinline__ double dual_residual(const double (&mx)[kRedWidth], double cinv) { return cinv * mx[kDualU]; }
+
+// after the last iteration without a decision: the test with 10x tolerances
+__device__ __forceinline__ int approximate_status(const ocp_b200_settings& S, const double (&mx)[kRedWidth], double cinv) {
+  const double ep = 10.0 * S.eps_abs + 10.0 * S.eps_rel * fmax(mx[kZU], mx[kAxU]);
+  const double ed = 10.0 * S.eps_abs + 10.0 * S.eps_rel * cinv * fmax(mx[kQU], fmax(mx[kAtyU], mx[kPxU]));
+  return prim_residual(mx) < ep && dual_residual(mx, cinv) < ed
+             ? OCP_B200_QP_SOLVED_INACCURATE : OCP_B200_QP_MAX_ITER_REACHED;
+}
+
+// check_termination: SOLVED, PRIMAL_INFEASIBLE or DUAL_INFEASIBLE, or -1 to continue
+template <class Ops>
+__device__ __forceinline__ int check_termination(const Ops& I, const QpVec& V, const ocp_b200_settings& S, Reducer& R,
+                                                 const double (&mx)[kRedWidth], double c, double cinv) {
+  const int tid = threadIdx.x, T = blockDim.x, n = V.n, m = V.m;
+  const double eps_prim = S.eps_abs + S.eps_rel * fmax(mx[kZU], mx[kAxU]);
+  const double eps_dual = S.eps_abs + S.eps_rel * cinv * fmax(mx[kQU], fmax(mx[kAtyU], mx[kPxU]));
+  const bool prim_ok = prim_residual(mx) < eps_prim, dual_ok = dual_residual(mx, cinv) < eps_dual;
+  bool prim_inf = false, dual_inf = false;
+  if (!prim_ok) {
+    // is_primal_infeasible: dy projected on the polar of the recession cone of [l, u]
+    double a2[1] = {0.0};
+    for (int i = tid; i < m; i += T) {
+      double dy = V.dy[i];
+      const double lo = V.l[i], hi = V.u[i];
+      if (hi > kInfty * kMinScaling) {
+        if (lo < -kInfty * kMinScaling) dy = 0.0; else dy = fmin(dy, 0.0);
+      } else if (lo < -kInfty * kMinScaling) {
+        dy = fmax(dy, 0.0);
+      }
+      V.dy[i] = dy;
+      a2[0] = fmax(a2[0], fabs(V.E[i] * dy));
+    }
+    // (the barrier of this reduction also orders the dy writes before the A' dy gather below)
+    block_reduce<1, true>(a2, R);
+    const double norm_dy = a2[0];
+    if (norm_dy > kDivisionTol) {
+      double lhs[1] = {0.0};
+      for (int i = tid; i < m; i += T) lhs[0] += V.u[i] * fmax(V.dy[i], 0.0) + V.l[i] * fmin(V.dy[i], 0.0);
+      block_reduce<1, false>(lhs, R);
+      if (lhs[0] < -S.eps_prim_inf * norm_dy) {
+        double na[1] = {0.0};
+        for (int j = tid; j < n; j += T) na[0] = fmax(na[0], fabs(I.col_dot_A(V.Aval, V.dy, j) / V.D[j]));
+        block_reduce<1, true>(na, R);
+        prim_inf = na[0] < S.eps_prim_inf * norm_dy;
+      }
+    }
+  }
+  if (!dual_ok) {
+    // is_dual_infeasible
+    double a2[1] = {0.0};
+    for (int j = tid; j < n; j += T) a2[0] = fmax(a2[0], fabs(V.D[j] * V.dx[j]));
+    block_reduce<1, true>(a2, R);
+    const double norm_dx = a2[0];
+    if (norm_dx > kDivisionTol) {
+      double qdx[1] = {0.0};
+      for (int j = tid; j < n; j += T) qdx[0] += V.q[j] * V.dx[j];
+      block_reduce<1, false>(qdx, R);
+      if (qdx[0] < -c * S.eps_dual_inf * norm_dx) {
+        double np_[1] = {0.0};
+        for (int j = tid; j < n; j += T) np_[0] = fmax(np_[0], fabs(I.col_dot_P(V.Pval, V.dx, j) / V.D[j]));
+        block_reduce<1, true>(np_, R);
+        if (np_[0] < c * S.eps_dual_inf * norm_dx) {
+          double viol[1] = {0.0};
+          I.for_rows_A(V.Aval, V.dx, [&](int i, double adx) {
+            const double a = adx / V.E[i];
+            if ((V.u[i] < kInfty * kMinScaling && a > S.eps_dual_inf * norm_dx) ||
+                (V.l[i] > -kInfty * kMinScaling && a < -S.eps_dual_inf * norm_dx)) viol[0] = 1.0;
+          });
+          block_reduce<1, true>(viol, R);
+          dual_inf = viol[0] == 0.0;
+        }
+      }
+    }
+  }
+  if (prim_ok && dual_ok) return OCP_B200_QP_SOLVED;
+  if (prim_inf) return OCP_B200_QP_PRIMAL_INFEASIBLE;
+  return dual_inf ? OCP_B200_QP_DUAL_INFEASIBLE : -1;
+}
+
+// adapt_rho: estimate from the SCALED residuals; true, with rho set to the estimate, when it moved by more
+// than adaptive_rho_tolerance (the caller then rebuilds its linear system)
+__device__ __forceinline__ bool adapt_rho(const ocp_b200_settings& S, const double (&mx)[kRedWidth], double& rho) {
+  const double pr = mx[kPrimS] / (fmax(mx[kZS], mx[kAxS]) + 1e-10);
+  const double dr = mx[kDualS] / (fmax(mx[kQS], fmax(mx[kAtyS], mx[kPxS])) + 1e-10);
+  double est = rho * sqrt(pr / (dr + 1e-10));
+  est = fmin(fmax(est, kRhoMin), kRhoMax);
+  if (!(est > rho * S.adaptive_rho_tolerance || est < rho / S.adaptive_rho_tolerance)) return false;
+  rho = est;
+  return true;
+}
+
+// one row of the check trace of instance 0: iteration, residuals, rho, linear solves so far, status of the check
+__device__ __forceinline__ void record_trace(const SolveArgs& A, int inst, int& n_trace, int iter, double prim_res,
+                                             double dual_res, double rho, int solves, int st) {
+  if (!(A.trace && inst == 0 && n_trace < A.max_trace)) return;
+  if (threadIdx.x == 0) {
+    double* tr = A.trace + size_t(n_trace) * OCP_B200_TRACE_WIDTH;
+    tr[0] = iter; tr[1] = prim_res; tr[2] = dual_res; tr[3] = rho; tr[4] = solves;
+    tr[5] = st < 0 ? OCP_B200_QP_UNSOLVED : st;
+  }
+  ++n_trace;
+}
+
+// store_solution: unscale in place (x <- D x, y <- E y / c), or NaN for a certificate
+__device__ __forceinline__ void store_solution(const QpVec& V, int status, double cinv) {
+  const bool has_sol = status != OCP_B200_QP_PRIMAL_INFEASIBLE && status != OCP_B200_QP_DUAL_INFEASIBLE;
+  const double nanv = __longlong_as_double(0x7ff8000000000000LL);
+  for (int j = threadIdx.x; j < V.n; j += blockDim.x) V.x[j] = has_sol ? V.D[j] * V.x[j] : nanv;
+  for (int i = threadIdx.x; i < V.m; i += blockDim.x) V.y[i] = has_sol ? cinv * V.E[i] * V.y[i] : nanv;
   __syncthreads();
 }
 

@@ -150,6 +150,17 @@ __device__ __forceinline__ void for_rows_A(const CompactIdx& C, const uint32_t* 
   }
 }
 
+// the sparse products of the OSQP layer (admm_common.cuh) over the templates and the arena
+struct CompactOps {
+  const CompactIdx& C;
+  const uint32_t* ar;
+  int m;
+  template <typename F>
+  __device__ __forceinline__ void for_rows_A(const double* Aval, const double* src, F f) const { compact::for_rows_A(C, ar, m, Aval, src, f); }
+  __device__ __forceinline__ double col_dot_A(const double* Aval, const double* v, int j) const { return compact::col_dot_A(C, ar, Aval, v, j); }
+  __device__ __forceinline__ double col_dot_P(const double* Pval, const double* v, int j) const { return compact::col_dot_P(C, ar, Pval, v, j); }
+};
+
 // ---------------------------------------------------------------------------------------
 // Tensor Memory as the home of the sweep blocks (BS = 16).
 //
@@ -547,10 +558,7 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
     const double e = W.E[i];
     const double lo = W.l[i] * e, hi = W.u[i] * e;
     W.l[i] = lo; W.u[i] = hi;
-    signed char ct = 0;
-    if (lo < -kInfty * kMinScaling && hi > kInfty * kMinScaling) ct = -1;
-    else if (hi - lo < kRhoTol) ct = 1;
-    W.ctype[i] = ct;
+    W.ctype[i] = constraint_type(lo, hi);
   }
   for (int k = tid; k < P.nnz_p; k += T) X.pslab[k] = X.psm[k];
   __syncthreads();
@@ -567,8 +575,8 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
   for (int i = tid; i < m; i += T) { W.z[i] = 0.0; W.y[i] = 0.0; W.w[i] = 0.0; }
   __syncthreads();
 
-  // OSQP without wall-clock profiling: 4 x check_termination, or ADAPTIVE_RHO_FIXED = 100 iterations when checks are off
-  const int rho_interval = S.adaptive_rho_interval > 0 ? S.adaptive_rho_interval : (S.check_termination > 0 ? 4 * S.check_termination : 100);
+  const CompactOps I{C, ar, m};
+  const int interval = rho_interval(S);
   int status = OCP_B200_QP_UNSOLVED, iter = 0, solves = 0, rho_updates = 0, checks = 0, n_trace = 0;
   double prim_res = 0.0, dual_res = 0.0;
   bool done = false;
@@ -587,10 +595,8 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
     clk.lap(OCP_B200_PHASE_SOLVE);
 
     // ---- x, z, y updates with relaxation and projection (update_x / update_z / update_y) ----
-    const bool can_check = S.check_termination > 0 && (iter % S.check_termination == 0);
-    const bool last_iter = iter == S.admm_max_iter;
-    const bool rho_time = S.adaptive_rho && rho_interval > 0 && (iter % rho_interval == 0);
-    const bool want_info = can_check || rho_time || last_iter;
+    const IterFlags F(S, interval, iter);
+    const bool want_info = F.want_info();
     {
       const uint32_t* tc = ar + C.arow.tent_off;
       const uint32_t* tp = ar + C.arow.tent2_off;
@@ -629,165 +635,48 @@ __device__ inline void solve_instance(const PatternDev& P, const CompactIdx& C, 
     clk.lap(OCP_B200_PHASE_UPDATE);
     if (!want_info) continue;
 
-    // ---- update_info: residuals of the unscaled problem ------------------------------------
+    // ---- update_info, check_termination, adapt_rho (admm_common.cuh) -------------------------
     ++checks;
+    const QpVec V = qp_vectors(W, n, m);
     double mx[kRedWidth];
-#pragma unroll
-    for (int k = 0; k < kRedWidth; ++k) mx[k] = 0.0;
-    for_rows_A(C, ar, m, W.Aval, W.x, [&](int i, double ax) {
-      const double einv = 1.0 / W.E[i];
-      const double zi = W.z[i];
-      const double rp = ax - zi;
-      mx[0] = fmax(mx[0], fabs(einv * rp));
-      mx[1] = fmax(mx[1], fabs(einv * ax));
-      mx[2] = fmax(mx[2], fabs(einv * zi));
-      mx[3] = fmax(mx[3], fabs(rp));
-      mx[4] = fmax(mx[4], fabs(ax));
-      mx[5] = fmax(mx[5], fabs(zi));
-    });
-    for (int j = tid; j < n; j += T) {
-      const double dinv = 1.0 / W.D[j];
-      const double qj = W.q[j];
-      const double px = col_dot_P(C, ar, W.Pval, W.x, j);
-      const double aty = col_dot_A(C, ar, W.Aval, W.y, j);
-      const double rd = qj + px + aty;
-      mx[6] = fmax(mx[6], fabs(dinv * rd));
-      mx[7] = fmax(mx[7], fabs(dinv * qj));
-      mx[8] = fmax(mx[8], fabs(dinv * px));
-      mx[9] = fmax(mx[9], fabs(dinv * aty));
-      mx[10] = fmax(mx[10], fabs(rd));
-      mx[11] = fmax(mx[11], fabs(qj));
-      mx[12] = fmax(mx[12], fabs(px));
-      mx[13] = fmax(mx[13], fabs(aty));
-    }
-    block_reduce<kRedWidth, true>(mx, R);
-    prim_res = mx[0];
-    dual_res = cinv * mx[6];
-
-    if (can_check || last_iter) {
-      // ---- check_termination ---------------------------------------------------------------
-      const double eps_prim = S.eps_abs + S.eps_rel * fmax(mx[2], mx[1]);
-      const double eps_dual = S.eps_abs + S.eps_rel * cinv * fmax(mx[7], fmax(mx[9], mx[8]));
-      const bool prim_ok = prim_res < eps_prim, dual_ok = dual_res < eps_dual;
-      bool prim_inf = false, dual_inf = false;
-      if (!prim_ok) {
-        // is_primal_infeasible: dy projected on the polar of the recession cone of [l, u]
-        double a2[1] = {0.0};
-        for (int i = tid; i < m; i += T) {
-          double dy = W.dy[i];
-          const double lo = W.l[i], hi = W.u[i];
-          if (hi > kInfty * kMinScaling) {
-            if (lo < -kInfty * kMinScaling) dy = 0.0; else dy = fmin(dy, 0.0);
-          } else if (lo < -kInfty * kMinScaling) {
-            dy = fmax(dy, 0.0);
-          }
-          W.dy[i] = dy;
-          a2[0] = fmax(a2[0], fabs(W.E[i] * dy));
-        }
-        block_reduce<1, true>(a2, R);
-        const double norm_dy = a2[0];
-        if (norm_dy > kDivisionTol) {
-          double lhs[1] = {0.0};
-          for (int i = tid; i < m; i += T) lhs[0] += W.u[i] * fmax(W.dy[i], 0.0) + W.l[i] * fmin(W.dy[i], 0.0);
-          block_reduce<1, false>(lhs, R);
-          if (lhs[0] < -S.eps_prim_inf * norm_dy) {
-            // A' dy gathers dy: the slab copy was written by other threads of this CTA
-            __syncthreads();
-            double na[1] = {0.0};
-            for (int j = tid; j < n; j += T) na[0] = fmax(na[0], fabs(col_dot_A(C, ar, W.Aval, W.dy, j) / W.D[j]));
-            block_reduce<1, true>(na, R);
-            prim_inf = na[0] < S.eps_prim_inf * norm_dy;
-          }
-        }
-      }
-      if (!dual_ok) {
-        // is_dual_infeasible
-        double a2[1] = {0.0};
-        for (int j = tid; j < n; j += T) a2[0] = fmax(a2[0], fabs(W.D[j] * W.dx[j]));
-        block_reduce<1, true>(a2, R);
-        const double norm_dx = a2[0];
-        if (norm_dx > kDivisionTol) {
-          double qdx[1] = {0.0};
-          for (int j = tid; j < n; j += T) qdx[0] += W.q[j] * W.dx[j];
-          block_reduce<1, false>(qdx, R);
-          if (qdx[0] < -c * S.eps_dual_inf * norm_dx) {
-            double np_[1] = {0.0};
-            for (int j = tid; j < n; j += T) np_[0] = fmax(np_[0], fabs(col_dot_P(C, ar, W.Pval, W.dx, j) / W.D[j]));
-            block_reduce<1, true>(np_, R);
-            if (np_[0] < c * S.eps_dual_inf * norm_dx) {
-              double viol[1] = {0.0};
-              for_rows_A(C, ar, m, W.Aval, W.dx, [&](int i, double adx) {
-                const double a = adx / W.E[i];
-                if ((W.u[i] < kInfty * kMinScaling && a > S.eps_dual_inf * norm_dx) ||
-                    (W.l[i] > -kInfty * kMinScaling && a < -S.eps_dual_inf * norm_dx)) viol[0] = 1.0;
-              });
-              block_reduce<1, true>(viol, R);
-              dual_inf = viol[0] == 0.0;
-            }
-          }
-        }
-      }
-      int st = -1;
-      if (prim_ok && dual_ok) st = OCP_B200_QP_SOLVED;
-      else if (prim_inf) st = OCP_B200_QP_PRIMAL_INFEASIBLE;
-      else if (dual_inf) st = OCP_B200_QP_DUAL_INFEASIBLE;
-      if (A.trace && inst == 0 && can_check && n_trace < A.max_trace) {
-        if (tid == 0) {
-          double* tr = A.trace + size_t(n_trace) * OCP_B200_TRACE_WIDTH;
-          tr[0] = iter; tr[1] = prim_res; tr[2] = dual_res; tr[3] = rho; tr[4] = solves;
-          tr[5] = st < 0 ? OCP_B200_QP_UNSOLVED : st;
-        }
-        ++n_trace;
-      }
+    update_info(I, V, R, mx);
+    prim_res = prim_residual(mx);
+    dual_res = dual_residual(mx, cinv);
+    if (F.can_check || F.last_iter) {
+      const int st = check_termination(I, V, S, R, mx, c, cinv);
+      if (F.can_check) record_trace(A, inst, n_trace, iter, prim_res, dual_res, rho, solves, st);
       if (st >= 0) { status = st; done = true; clk.lap(OCP_B200_PHASE_CHECK); continue; }
-      if (last_iter) {
-        // approximate termination test with 10x tolerances, then MAX_ITER_REACHED
-        const double ep = 10.0 * S.eps_abs + 10.0 * S.eps_rel * fmax(mx[2], mx[1]);
-        const double ed = 10.0 * S.eps_abs + 10.0 * S.eps_rel * cinv * fmax(mx[7], fmax(mx[9], mx[8]));
-        status = (prim_res < ep && dual_res < ed) ? OCP_B200_QP_SOLVED_INACCURATE : OCP_B200_QP_MAX_ITER_REACHED;
-        done = true;
-        continue;
-      }
+      if (F.last_iter) { status = approximate_status(S, mx, cinv); done = true; continue; }
     }
-
-    if (rho_time) {
-      // ---- adapt_rho: estimate from SCALED residuals, applied when it moved by > tolerance
-      const double pr = mx[3] / (fmax(mx[5], mx[4]) + 1e-10);
-      const double dr = mx[10] / (fmax(mx[11], fmax(mx[13], mx[12])) + 1e-10);
-      double est = rho * sqrt(pr / (dr + 1e-10));
-      est = fmin(fmax(est, kRhoMin), kRhoMax);
-      if (est > rho * S.adaptive_rho_tolerance || est < rho / S.adaptive_rho_tolerance) {
-        rho = est;
-        ++rho_updates;
-        rv = Rho(rho);
-        // the factorisation works in the space of the iteration vectors: park x, z, y in the slab
-        // (element i written and read back by the same thread)
-        __syncthreads();
-        for (int j = tid; j < n; j += T) X.sx[j] = W.x[j];
-        for (int i = tid; i < m; i += T) { X.sz[i] = W.z[i]; X.sy[i] = W.y[i]; }
-        __syncthreads();
-        // (inlined a second time on purpose: an out-of-line copy shared with the set-up was measured slower,
-        // 9.6 -> 9.8 ms per launch with P and W passed by value, 11.7 ms by reference)
-        direct::tri_assemble_program(P, W, rv, sigma);
-        direct::tri_factor_twisted<BS, true, true, BS == 16>(P, W);
-        if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
-        for (int j = tid; j < n; j += T) W.x[j] = X.sx[j];
-        for (int i = tid; i < m; i += T) {
-          const double zi = X.sz[i], yi = X.sy[i];
-          W.z[i] = zi; W.y[i] = yi;
-          W.w[i] = rv.of(W.ctype[i]) * zi - yi;
-        }
-        __syncthreads();
+    if (F.rho_time && adapt_rho(S, mx, rho)) {
+      ++rho_updates;
+      rv = Rho(rho);
+      // the factorisation works in the space of the iteration vectors: park x, z, y in the slab
+      // (element i written and read back by the same thread)
+      __syncthreads();
+      for (int j = tid; j < n; j += T) X.sx[j] = W.x[j];
+      for (int i = tid; i < m; i += T) { X.sz[i] = W.z[i]; X.sy[i] = W.y[i]; }
+      __syncthreads();
+      // (inlined a second time on purpose: an out-of-line copy shared with the set-up was measured slower,
+      // 9.6 -> 9.8 ms per launch with P and W passed by value, 11.7 ms by reference)
+      direct::tri_assemble_program(P, W, rv, sigma);
+      direct::tri_factor_twisted<BS, true, true, BS == 16>(P, W);
+      if constexpr (BS == 16) tmem_publish<BS>(W, P.tri_nb, tmem);
+      for (int j = tid; j < n; j += T) W.x[j] = X.sx[j];
+      for (int i = tid; i < m; i += T) {
+        const double zi = X.sz[i], yi = X.sy[i];
+        W.z[i] = zi; W.y[i] = yi;
+        W.w[i] = rv.of(W.ctype[i]) * zi - yi;
       }
+      __syncthreads();
     }
     clk.lap(OCP_B200_PHASE_CHECK);
   }
-  if (!done) { status = OCP_B200_QP_MAX_ITER_REACHED; }
+  if (!done) status = OCP_B200_QP_MAX_ITER_REACHED;
   if (A.trace && inst == 0 && tid == 0 && A.n_trace) *A.n_trace = n_trace;
-  const int iters_done = done ? iter - 1 : S.admm_max_iter;
-  out = QpResult{status, iters_done, solves, rho_updates, checks, prim_res, dual_res, rho};
-
-  // ---- store_solution: unscale in place (x <- D x, y <- E y / c), or NaN for a certificate
+  out = QpResult{status, done ? iter - 1 : S.admm_max_iter, solves, rho_updates, checks, prim_res, dual_res, rho};
+  // store_solution (admm_common.cuh), written out here: the shared function, same arithmetic, costs the BS = 20
+  // instantiation 16 + 48 bytes of spill stores / loads more (register allocation at the 128 cap, DESIGN.md 5.5)
   const bool has_sol = status != OCP_B200_QP_PRIMAL_INFEASIBLE && status != OCP_B200_QP_DUAL_INFEASIBLE;
   const double nanv = __longlong_as_double(0x7ff8000000000000LL);
   for (int j = tid; j < n; j += T) W.x[j] = has_sol ? W.D[j] * W.x[j] : nanv;
@@ -838,12 +727,7 @@ admm_compact_kernel(const PatternDev P, const CompactIdx C, const ocp_b200_setti
   Ctx X{ar, sm + L.rscale, sm + L.psm, gl + L.an, gl + L.cn, gl + L.sx, gl + L.sz, gl + L.sy, gl + L.pval};
   __syncthreads();
   Reducer R{red_buf, 0, (kThreads / 32) * kRedWidth};
-  while (true) {
-    if (threadIdx.x == 0) s_inst = atomicAdd(A.counter, 1);
-    __syncthreads();
-    const int inst = s_inst;
-    __syncthreads();
-    if (inst >= A.B) break;
+  for (int inst; (inst = next_instance(A, s_inst)) < A.B;) {
     QpResult res;
     solve_instance<BS>(P, C, S, A, W, X, R, inst, res, tmem);
     write_outputs(P, A, W.x, W.y, R, inst, res);

@@ -1217,10 +1217,7 @@ __device__ inline void solve_instance(const PatternDev& P, const ocp_b200_settin
   for (int i = tid; i < m; i += T) {
     const double lo = W.l[i] * W.E[i], hi = W.u[i] * W.E[i];
     W.l[i] = lo; W.u[i] = hi;
-    signed char ct = 0;
-    if (lo < -kInfty * kMinScaling && hi > kInfty * kMinScaling) ct = -1;
-    else if (hi - lo < kRhoTol) ct = 1;
-    W.ctype[i] = ct;
+    W.ctype[i] = constraint_type(lo, hi);
   }
   __syncthreads();
   Rho rv(rho);
@@ -1230,8 +1227,8 @@ __device__ inline void solve_instance(const PatternDev& P, const ocp_b200_settin
   factor_dispatch<kPlace>(P, W);
   clk.lap(OCP_B200_PHASE_FACTOR);
 
-  // OSQP without wall-clock profiling: 4 x check_termination, or ADAPTIVE_RHO_FIXED = 100 iterations when checks are off
-  const int rho_interval = S.adaptive_rho_interval > 0 ? S.adaptive_rho_interval : (S.check_termination > 0 ? 4 * S.check_termination : 100);
+  const PatternOps I{P};
+  const int interval = rho_interval(S);
   int status = OCP_B200_QP_UNSOLVED, iter = 0, solves = 0, rho_updates = 0, checks = 0, n_trace = 0;
   double prim_res = 0.0, dual_res = 0.0;
   bool done = false;
@@ -1249,10 +1246,8 @@ __device__ inline void solve_instance(const PatternDev& P, const ocp_b200_settin
     clk.lap(OCP_B200_PHASE_SOLVE);
 
     // ---- x, z, y updates with relaxation and projection (update_x / update_z / update_y) ----
-    const bool can_check = S.check_termination > 0 && (iter % S.check_termination == 0);
-    const bool last_iter = iter == S.admm_max_iter;
-    const bool rho_time = S.adaptive_rho && rho_interval > 0 && (iter % rho_interval == 0);
-    const bool want_info = can_check || rho_time || last_iter;
+    const IterFlags F(S, interval, iter);
+    const bool want_info = F.want_info();
     for_rows_A(P, W.Aval, W.b, [&](int i, double zt) {
       const signed char ct = W.ctype[i];
       const double rh = rv.of(ct);
@@ -1275,151 +1270,32 @@ __device__ inline void solve_instance(const PatternDev& P, const ocp_b200_settin
     clk.lap(OCP_B200_PHASE_UPDATE);
     if (!want_info) continue;
 
-    // ---- update_info: residuals of the unscaled problem ------------------------------------
+    // ---- update_info, check_termination, adapt_rho (admm_common.cuh) -------------------------
     ++checks;
+    const QpVec V = qp_vectors(W, n, m);
     double mx[kRedWidth];
-#pragma unroll
-    for (int k = 0; k < kRedWidth; ++k) mx[k] = 0.0;
-    for_rows_A(P, W.Aval, W.x, [&](int i, double ax) {
-      const double einv = 1.0 / W.E[i];
-      const double zi = W.z[i];
-      const double rp = ax - zi;
-      mx[0] = fmax(mx[0], fabs(einv * rp));
-      mx[1] = fmax(mx[1], fabs(einv * ax));
-      mx[2] = fmax(mx[2], fabs(einv * zi));
-      mx[3] = fmax(mx[3], fabs(rp));
-      mx[4] = fmax(mx[4], fabs(ax));
-      mx[5] = fmax(mx[5], fabs(zi));
-    });
-    for (int j = tid; j < n; j += T) {
-      const double dinv = 1.0 / W.D[j];
-      const double px = col_dot_P(P, W.Pval, W.x, j);
-      const double aty = col_dot_A(P, W.Aval, W.y, j);
-      const double rd = W.q[j] + px + aty;
-      mx[6] = fmax(mx[6], fabs(dinv * rd));
-      mx[7] = fmax(mx[7], fabs(dinv * W.q[j]));
-      mx[8] = fmax(mx[8], fabs(dinv * px));
-      mx[9] = fmax(mx[9], fabs(dinv * aty));
-      mx[10] = fmax(mx[10], fabs(rd));
-      mx[11] = fmax(mx[11], fabs(W.q[j]));
-      mx[12] = fmax(mx[12], fabs(px));
-      mx[13] = fmax(mx[13], fabs(aty));
-    }
-    block_reduce<kRedWidth, true>(mx, R);
-    prim_res = mx[0];
-    dual_res = cinv * mx[6];
-
-    if (can_check || last_iter) {
-      // ---- check_termination ---------------------------------------------------------------
-      const double eps_prim = S.eps_abs + S.eps_rel * fmax(mx[2], mx[1]);
-      const double eps_dual = S.eps_abs + S.eps_rel * cinv * fmax(mx[7], fmax(mx[9], mx[8]));
-      const bool prim_ok = prim_res < eps_prim, dual_ok = dual_res < eps_dual;
-      bool prim_inf = false, dual_inf = false;
-      if (!prim_ok) {
-        // is_primal_infeasible: dy projected on the polar of the recession cone of [l, u]
-        double a2[1] = {0.0};
-        for (int i = tid; i < m; i += T) {
-          double dy = W.dy[i];
-          if (W.u[i] > kInfty * kMinScaling) {
-            if (W.l[i] < -kInfty * kMinScaling) dy = 0.0; else dy = fmin(dy, 0.0);
-          } else if (W.l[i] < -kInfty * kMinScaling) {
-            dy = fmax(dy, 0.0);
-          }
-          W.dy[i] = dy;
-          a2[0] = fmax(a2[0], fabs(W.E[i] * dy));
-        }
-        block_reduce<1, true>(a2, R);
-        const double norm_dy = a2[0];
-        if (norm_dy > kDivisionTol) {
-          double lhs[1] = {0.0};
-          for (int i = tid; i < m; i += T) lhs[0] += W.u[i] * fmax(W.dy[i], 0.0) + W.l[i] * fmin(W.dy[i], 0.0);
-          block_reduce<1, false>(lhs, R);
-          if (lhs[0] < -S.eps_prim_inf * norm_dy) {
-            double na[1] = {0.0};
-            for (int j = tid; j < n; j += T) na[0] = fmax(na[0], fabs(col_dot_A(P, W.Aval, W.dy, j) / W.D[j]));
-            block_reduce<1, true>(na, R);
-            prim_inf = na[0] < S.eps_prim_inf * norm_dy;
-          }
-        }
-      }
-      if (!dual_ok) {
-        // is_dual_infeasible
-        double a2[1] = {0.0};
-        for (int j = tid; j < n; j += T) a2[0] = fmax(a2[0], fabs(W.D[j] * W.dx[j]));
-        block_reduce<1, true>(a2, R);
-        const double norm_dx = a2[0];
-        if (norm_dx > kDivisionTol) {
-          double qdx[1] = {0.0};
-          for (int j = tid; j < n; j += T) qdx[0] += W.q[j] * W.dx[j];
-          block_reduce<1, false>(qdx, R);
-          if (qdx[0] < -c * S.eps_dual_inf * norm_dx) {
-            double np_[1] = {0.0};
-            for (int j = tid; j < n; j += T) np_[0] = fmax(np_[0], fabs(col_dot_P(P, W.Pval, W.dx, j) / W.D[j]));
-            block_reduce<1, true>(np_, R);
-            if (np_[0] < c * S.eps_dual_inf * norm_dx) {
-              double viol[1] = {0.0};
-              for_rows_A(P, W.Aval, W.dx, [&](int i, double adx) {
-                const double a = adx / W.E[i];
-                if ((W.u[i] < kInfty * kMinScaling && a > S.eps_dual_inf * norm_dx) ||
-                    (W.l[i] > -kInfty * kMinScaling && a < -S.eps_dual_inf * norm_dx)) viol[0] = 1.0;
-              });
-              block_reduce<1, true>(viol, R);
-              dual_inf = viol[0] == 0.0;
-            }
-          }
-        }
-      }
-      int st = -1;
-      if (prim_ok && dual_ok) st = OCP_B200_QP_SOLVED;
-      else if (prim_inf) st = OCP_B200_QP_PRIMAL_INFEASIBLE;
-      else if (dual_inf) st = OCP_B200_QP_DUAL_INFEASIBLE;
-      if (A.trace && inst == 0 && can_check && n_trace < A.max_trace) {
-        if (tid == 0) {
-          double* tr = A.trace + size_t(n_trace) * OCP_B200_TRACE_WIDTH;
-          tr[0] = iter; tr[1] = prim_res; tr[2] = dual_res; tr[3] = rho; tr[4] = solves;
-          tr[5] = st < 0 ? OCP_B200_QP_UNSOLVED : st;
-        }
-        ++n_trace;
-      }
+    update_info(I, V, R, mx);
+    prim_res = prim_residual(mx);
+    dual_res = dual_residual(mx, cinv);
+    if (F.can_check || F.last_iter) {
+      const int st = check_termination(I, V, S, R, mx, c, cinv);
+      if (F.can_check) record_trace(A, inst, n_trace, iter, prim_res, dual_res, rho, solves, st);
       if (st >= 0) { status = st; done = true; clk.lap(OCP_B200_PHASE_CHECK); continue; }
-      if (last_iter) {
-        // approximate termination test with 10x tolerances, then MAX_ITER_REACHED
-        const double ep = 10.0 * S.eps_abs + 10.0 * S.eps_rel * fmax(mx[2], mx[1]);
-        const double ed = 10.0 * S.eps_abs + 10.0 * S.eps_rel * cinv * fmax(mx[7], fmax(mx[9], mx[8]));
-        status = (prim_res < ep && dual_res < ed) ? OCP_B200_QP_SOLVED_INACCURATE : OCP_B200_QP_MAX_ITER_REACHED;
-        done = true;
-        continue;
-      }
+      if (F.last_iter) { status = approximate_status(S, mx, cinv); done = true; continue; }
     }
-
-    if (rho_time) {
-      // ---- adapt_rho: estimate from SCALED residuals, applied when it moved by > tolerance
-      const double pr = mx[3] / (fmax(mx[5], mx[4]) + 1e-10);
-      const double dr = mx[10] / (fmax(mx[11], fmax(mx[13], mx[12])) + 1e-10);
-      double est = rho * sqrt(pr / (dr + 1e-10));
-      est = fmin(fmax(est, kRhoMin), kRhoMax);
-      if (est > rho * S.adaptive_rho_tolerance || est < rho / S.adaptive_rho_tolerance) {
-        rho = est;
-        ++rho_updates;
-        rv = Rho(rho);
-        for (int i = tid; i < m; i += T) W.w[i] = rv.of(W.ctype[i]) * W.z[i] - W.y[i];
-        tri_assemble(P, W, rv, sigma);
-        factor_dispatch<kPlace>(P, W);
-      }
+    if (F.rho_time && adapt_rho(S, mx, rho)) {
+      ++rho_updates;
+      rv = Rho(rho);
+      for (int i = tid; i < m; i += T) W.w[i] = rv.of(W.ctype[i]) * W.z[i] - W.y[i];
+      tri_assemble(P, W, rv, sigma);
+      factor_dispatch<kPlace>(P, W);
     }
     clk.lap(OCP_B200_PHASE_CHECK);
   }
-  if (!done) { status = OCP_B200_QP_MAX_ITER_REACHED; }
+  if (!done) status = OCP_B200_QP_MAX_ITER_REACHED;
   if (A.trace && inst == 0 && tid == 0 && A.n_trace) *A.n_trace = n_trace;
-  const int iters_done = done ? iter - 1 : S.admm_max_iter;
-  out = QpResult{status, iters_done, solves, rho_updates, checks, prim_res, dual_res, rho};
-
-  // ---- store_solution: unscale in place (x <- D x, y <- E y / c), or NaN for a certificate
-  const bool has_sol = status != OCP_B200_QP_PRIMAL_INFEASIBLE && status != OCP_B200_QP_DUAL_INFEASIBLE;
-  const double nanv = __longlong_as_double(0x7ff8000000000000LL);
-  for (int j = tid; j < n; j += T) W.x[j] = has_sol ? W.D[j] * W.x[j] : nanv;
-  for (int i = tid; i < m; i += T) W.y[i] = has_sol ? cinv * W.E[i] * W.y[i] : nanv;
-  __syncthreads();
+  out = QpResult{status, done ? iter - 1 : S.admm_max_iter, solves, rho_updates, checks, prim_res, dual_res, rho};
+  store_solution(qp_vectors(W, n, m), status, cinv);
 }
 
 // persistent kernel: CTAs pull instances from A.counter
@@ -1458,12 +1334,7 @@ admm_direct_kernel(const PatternDev P, const ocp_b200_settings S, const SolveArg
     __syncthreads();
   }
   Reducer R{red_buf, 0, (kThreads / 32) * kRedWidth};
-  while (true) {
-    if (threadIdx.x == 0) s_inst = atomicAdd(A.counter, 1);
-    __syncthreads();
-    const int inst = s_inst;
-    __syncthreads();
-    if (inst >= A.B) break;
+  for (int inst; (inst = next_instance(A, s_inst)) < A.B;) {
     QpResult res;
     solve_instance<kPlace>(PL, S, A, W, R, inst, res);
     write_outputs(P, A, W.x, W.y, R, inst, res);

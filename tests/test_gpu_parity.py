@@ -237,17 +237,38 @@ def test_reference_kat_cases_on_gpu(native, case):
     assert np.abs(x2 - expected).max() < 1e-6
 
 
-def test_infeasible_qp_reports_certificate(native):
-    """x in [0,1] with the row x >= 2: primal infeasible -> status 3 and a NaN solution, which the
-    reference adds to its iterate unchecked (SURVEY.md §3.3)."""
+def _check_certificates(native, settings):
+    """Primal: x in [0,1] with the row x >= 2 -> status 3 and a NaN solution, which the reference adds to its
+    iterate unchecked (SURVEY.md §3.3).  Dual: min -x with x >= 0 and no curvature (empty H) -> status 5."""
     hc, hr = [0, 1], [0]
     ac, ar = [0, 2], [0, 1]
-    sol = native.Solver.create(1, 2, hc, hr, ac, ar)
+    sol = native.Solver.create(1, 2, hc, hr, ac, ar, settings=settings)
     x, y, info = sol.qp_solve_batch(np.array([[1.0]]), np.array([[0.0]]), np.array([[1.0, 1.0]]),
                                     np.array([[0.0, 2.0]]), np.array([[1.0, 3.0]]))
     ox, oy, oinfo, _ = _oracle.qp_solve(1, 2, hc, hr, [1.0], [0.0], ac, ar, [1.0, 1.0], [0.0, 2.0], [1.0, 3.0])
     assert info[0, 0] == oinfo[0] == native.QP_PRIMAL_INFEASIBLE
     assert np.isnan(x).all() and np.isnan(ox).all()
+    hc, hr = [0, 0], []
+    ac, ar = [0, 1], [0]
+    sol = native.Solver.create(1, 1, hc, hr, ac, ar, settings=settings)
+    x, y, info = sol.qp_solve_batch(np.zeros((1, 0)), np.array([[-1.0]]), np.array([[1.0]]),
+                                    np.array([[0.0]]), np.array([[np.inf]]))
+    ox, oy, oinfo, _ = _oracle.qp_solve(1, 1, hc, hr, [], [-1.0], ac, ar, [1.0], [0.0], [np.inf])
+    assert info[0, 0] == oinfo[0] == native.QP_DUAL_INFEASIBLE
+    assert np.isnan(x).all() and np.isnan(ox).all()
+
+
+def test_infeasible_qp_reports_certificate(native):
+    """Both certificates on the direct kernel (the default preconditioner, BLOCK_TRIDIAG)."""
+    _check_certificates(native, native.default_settings())
+
+
+@pytest.mark.parametrize("precond", [0, 1])
+def test_infeasible_qp_reports_certificate_on_pcg(native, precond):
+    """Both certificates on the PCG kernel (DIAGONAL and BLOCK_JACOBI preconditioners)."""
+    s = native.default_settings()
+    s.pcg_precond = precond
+    _check_certificates(native, s)
 
 
 def test_class_api_single_instance(problems, native):
@@ -543,8 +564,8 @@ def test_launch_plans_of_the_headline_shape(problems, native):
 
 
 def test_compact_plan_qp_level(native, monkeypatch):
-    """QP-level entry points on the compact kernel: primal / dual solutions, residuals, the check trace, an
-    infeasible QP (certificate -> NaN solution) and inconsistent bounds (zero step)."""
+    """QP-level entry points on the compact kernel: primal / dual solutions, residuals, the check trace, a primal
+    and a dual infeasible QP (certificate -> NaN solution) and inconsistent bounds (zero step)."""
     monkeypatch.setenv("OCP_B200_PLAN", "compact")
     prob = native.Problem("quadrotor")
     ora = _oracle.OracleProblem("quadrotor")
@@ -579,6 +600,19 @@ def test_compact_plan_qp_level(native, monkeypatch):
         assert info2[b, native.INFO["status"]] == oinfo[0] == native.QP_PRIMAL_INFEASIBLE
         assert info2[b, native.INFO["iters"]] == oinfo[1]
         assert np.array_equal(np.isnan(x2[b]), np.isnan(ox))
+    # dual infeasible: no curvature, and the first rotor input of the last stage (rows 0..n-1 of A bound the
+    # variables) released, so the linear cost decreases without limit along it.  The iterates grow without bound
+    # here, and so do the rounding differences between the two linear solves: the certificate is the same, the
+    # check at which it fires need not be.
+    h4, l4, u4 = np.zeros_like(hv), l.copy(), u.copy()
+    row = prob.n - 4
+    l4[:, row], u4[:, row] = -np.inf, np.inf
+    x4, y4, info4 = prob.solver.qp_solve_batch(h4, q, av, l4, u4)
+    for b in range(hv.shape[0]):
+        ox, oy, oinfo, _ = _oracle.qp_solve(prob.n, prob.m, prob.h_colptr, prob.h_rowidx, h4[b], q[b], prob.a_colptr,
+                                            prob.a_rowidx, av[b], l4[b], u4[b], settings=sv)
+        assert info4[b, native.INFO["status"]] == oinfo[0] == native.QP_DUAL_INFEASIBLE
+        assert np.isnan(x4[b]).all() and np.isnan(ox).all()
     # l > u: osqp_setup refuses, zero step
     l3 = l.copy(); l3[:, 5] = u[:, 5] + 1.0
     x3, y3, info3 = prob.solver.qp_solve_batch(hv, q, av, l3, u)
