@@ -1,9 +1,11 @@
 """GPU parity tests proper: the CUDA path, called through the C ABI (include/ocp_b200.h), against
 the CPU oracle on the same seeded inputs.
 
-Tolerances (FP64 on both sides; the GPU solves the reduced KKT system with PCG to a relative
-residual of 1e-10 where the oracle uses an exact LDL' solve, so ADMM iterates agree to rounding
-amplified by the conditioning of the scaled KKT system):
+Tolerances (FP64 on both sides; by default the GPU factorises the reduced KKT system P + sigma I +
+A' diag(rho) A directly (bordered block-tridiagonal LDL', admm_direct_kernel.cuh / admm_compact_kernel.cuh;
+PCG to a relative residual of pcg_tol = 1e-10 where that structure is absent) where the oracle uses
+an exact LDL' solve of the full KKT system, so ADMM iterates agree to rounding amplified by the
+conditioning of the scaled KKT system):
   * sparsity patterns / CSC index arrays: bit-exact;
   * local-system values (H, grad, J, l - c, u - c): 1e-12 relative;
   * QP primal / dual solutions, SQP iterates: 1e-6 relative to the vector's inf-norm
