@@ -12,7 +12,10 @@
 // it with s = e_j, so lane j ends up holding column j of the Jacobian / Hessian block --
 // the same straight-line code on every lane, no divergence.  Lanes scatter their column
 // into a shared-memory image of the group's CONTIGUOUS CSC value range and the warp then
-// streams that range to HBM with coalesced 16-byte stores.  Programs that are textually
+// streams that range to HBM with coalesced 16-byte stores.  A group whose image exceeds a
+// fixed budget (the p group at long horizons: its Hessian range holds one entry per stage
+// and parameter) skips the image and stores straight into the instance's rows, so the
+// kernel's static shared memory does not depend on the horizon.  Programs that are textually
 // identical after making variable indices stage-relative are emitted once (all interior
 // stages of an OCP share one template).
 #include "optimal_control_problem/codegen/StageCodegen.h"
@@ -136,11 +139,18 @@ unsigned long long fnv1a(const std::string& s) {
 struct GroupPlan {
   int first_col = 0, ncols = 0, xoff = 0;  // xoff: offset of the X base pointer into x
   bool is_p = false;
+  bool staged = true;   // image in shared memory + copy_out; false: lanes store straight to global memory
   int tmpl = -1, otmpl = -1;
   int a_base = 0, a_len = 0, h_base = 0, h_len = 0;
   int atab_off = 0, htab_off = 0, ctab_off = 0;
   int n_tg = 0, n_th = 0, n_cown = 0;
 };
+
+// Largest per-unit image (A range + H range of a group, doubles) that is staged in shared memory.  It holds every
+// group of the three benchmark models at H = 20; a block's images then stay under 4 units x 2 x 640 doubles = 40 KB.
+constexpr int kStageBudget = 640;
+// c_groups (12 ints per group, 13 with the `staged` flag) lives in the 64 KB __constant__ bank
+constexpr size_t kConstantBank = 64 * 1024;
 
 void int_array(std::ostringstream& os, const char* decl, const std::vector<int>& v) {
   os << decl << "[" << std::max<size_t>(v.size(), 1) << "] = {";
@@ -202,7 +212,15 @@ ModelSource generate(const ModelSpec& spec) {
   for (GroupPlan& g : groups) {
     g.a_base = ac[g.first_col]; g.a_len = ac[g.first_col + g.ncols] - g.a_base;
     g.h_base = hc[g.first_col]; g.h_len = hc[g.first_col + g.ncols] - g.h_base;
+    g.staged = g.a_len + g.h_len <= kStageBudget;
   }
+  const bool any_direct = std::any_of(groups.begin(), groups.end(), [](const GroupPlan& g) { return !g.staged; });
+  const size_t group_info_bytes = (any_direct ? 13 : 12) * sizeof(int);
+  casadi_assert(G * group_info_bytes <= kConstantBank,
+                "codegen: " + std::to_string(G) + " column groups (horizon " + std::to_string(H) +
+                    ") overflow the 64 KB constant bank that holds the group table (" +
+                    std::to_string(group_info_bytes) + " bytes per group, at most " +
+                    std::to_string(kConstantBank / group_info_bytes) + " groups)");
 
   // ---- dependencies of g rows and gradient entries on w --------------------------------------
   std::vector<SXElem> roots;
@@ -253,6 +271,7 @@ ModelSource generate(const ModelSpec& spec) {
   // ---- per group: tangent program, tables, text; de-duplicate text ---------------------
   std::vector<int> tab;                       // all int tables, concatenated
   std::vector<std::string> tmpl_text, otmpl_text;
+  std::vector<bool> tmpl_staged;
   std::unordered_map<std::string, int> tmpl_index, otmpl_index;
   size_t nstmt_total = 0;
   int stage_a = 1, stage_h = 1;
@@ -269,12 +288,10 @@ ModelSource generate(const ModelSpec& spec) {
   // quadrotor has 16-column groups: one unit per warp leaves half the lanes idle.
   int maxcols = 1;
   for (const GroupPlan& gp : groups) maxcols = std::max(maxcols, gp.ncols);
-  int max_image = 1;   // doubles of the largest per-unit shared-memory image (A range + H range of a group)
-  {
-    int ma = 0, mh = 0;
-    for (const GroupPlan& gp : groups) { ma = std::max(ma, gp.a_len); mh = std::max(mh, gp.h_len); }
-    max_image = std::max(1, ma + mh);
-  }
+  int max_image = 1;   // doubles of the per-unit shared-memory image (largest A range + H range of a staged group)
+  for (const GroupPlan& gp : groups)
+    if (gp.staged) { stage_a = std::max(stage_a, gp.a_len); stage_h = std::max(stage_h, gp.h_len); }
+  max_image = stage_a + stage_h;
   int L = 32;
   // (4 warps per block, static shared memory: keep the images of a block under 40 KB)
   while (L > 8 && L / 2 >= maxcols && size_t(4) * (32 / (L / 2)) * max_image * sizeof(double) <= 40 * 1024) L /= 2;
@@ -285,8 +302,6 @@ ModelSource generate(const ModelSpec& spec) {
 
   for (int gidx = 0; gidx < G; ++gidx) {
     GroupPlan& g = groups[gidx];
-    stage_a = std::max(stage_a, g.a_len);
-    stage_h = std::max(stage_h, g.h_len);
     const int nd = g.ncols;
     std::vector<SXElem> V(w.begin() + g.first_col, w.begin() + g.first_col + nd), seeds;
     for (int j = 0; j < nd; ++j) seeds.push_back(SXElem::sym("seed" + std::to_string(j)));
@@ -322,6 +337,7 @@ ModelSource generate(const ModelSpec& spec) {
     Emitter em;
     leaf_names(em, g, &seeds);
     std::ostringstream t;
+    if (!g.staged) t << "  // sA / sH point into global memory (the group's image exceeds the shared-memory budget)\n";
     t << "  // tangent directions: " << nd << ", g-row tangents: " << g.n_tg << ", gradient tangents: "
       << g.n_th << ", owned g rows: " << g.n_cown << "\n";
     t << "  const bool act = dir < " << nd << ";\n  const int dsel = act ? dir : 0;\n";
@@ -365,6 +381,7 @@ ModelSource generate(const ModelSpec& spec) {
       g.tmpl = static_cast<int>(tmpl_text.size());
       tmpl_index[text] = g.tmpl;
       tmpl_text.push_back(text);
+      tmpl_staged.push_back(g.staged);
       nstmt_total += em.nstmt;
     } else {
       g.tmpl = it->second;
@@ -398,6 +415,9 @@ ModelSource generate(const ModelSpec& spec) {
     << "  n=" << n << " m=" << m << " nnz(H)=" << hr.size() << " nnz(A)=" << ar.size() << "\n";
   s << "// groups: " << G << ", stage templates: " << tmpl_text.size() << ", objective templates: "
     << otmpl_text.size() << "\n";
+  const int num_direct = static_cast<int>(std::count_if(groups.begin(), groups.end(), [](const GroupPlan& g) { return !g.staged; }));
+  s << "// unit lanes: " << L << ", groups storing straight to global memory: " << num_direct
+    << ", static shared memory of assemble_kernel: " << 4 * (32 / L) * (stage_a + stage_h) * sizeof(double) << " bytes\n";
   s << "#include <cuda_runtime.h>\n#include <math_constants.h>\n#include \"ocp_b200_model.h\"\n\n";
   s << "#define OCP_INF CUDART_INF\n#define OCP_NAN CUDART_NAN\n\nnamespace {\n";
   s << "constexpr int NP = " << np << ", NF = " << nf << ", HORIZON = " << H << ", NG = " << ng << ";\n";
@@ -410,12 +430,12 @@ ModelSource generate(const ModelSpec& spec) {
   s << "constexpr int WARPS_PER_BLOCK = 4, MIN_BLOCKS = " << min_blocks << ";\n";
   s << "constexpr int UNIT_LANES = " << L << ", UNITS_PER_WARP = 32 / UNIT_LANES;   // lanes per (instance, group) unit\n\n";
   s << "struct GroupInfo { int tmpl, otmpl, first_col, ncols, xoff, a_base, a_len, h_base, h_len, atab_off, "
-       "htab_off, ctab_off; };\n";
+       "htab_off, ctab_off" << (any_direct ? ", staged" : "") << "; };\n";
   s << "__constant__ GroupInfo c_groups[NUM_GROUPS] = {\n";
   for (const GroupPlan& g : groups)
     s << "  {" << g.tmpl << "," << g.otmpl << "," << g.first_col << "," << g.ncols << "," << g.xoff << ","
       << g.a_base << "," << g.a_len << "," << g.h_base << "," << g.h_len << "," << g.atab_off << ","
-      << g.htab_off << "," << g.ctab_off << "},\n";
+      << g.htab_off << "," << g.ctab_off << (any_direct ? (g.staged ? ",1" : ",0") : "") << "},\n";
   s << "};\n";
   int_array(s, "__device__ const int d_tab", tab);
   int_array(s, "__device__ const int d_acol", ac);
@@ -476,11 +496,17 @@ assemble_kernel(const int B, const double* __restrict__ x, const double* __restr
   double* li = l + static_cast<size_t>(inst) * ldm;
   double* ui = u + static_cast<size_t>(inst) * ldm;
   double* qi = q + static_cast<size_t>(inst) * ldn;
-  // identity rows of c = [p; x; g]: A entry 1, bounds l - w, u - w (first frame pinned to `frames`)
+)";
+  if (any_direct)
+    s << R"(  double* gA = av + static_cast<size_t>(inst) * lda + gi.a_base;   // groups that skip the shared-memory image
+  double* gH = hv + static_cast<size_t>(inst) * ldh + gi.h_base;
+)";
+  s << R"(  // identity rows of c = [p; x; g]: A entry 1, bounds l - w, u - w (first frame pinned to `frames`)
   for (int j = lane; valid && j < gi.ncols; j += UNIT_LANES) {
     const int col = gi.first_col + j;
-    sA[d_acol[col] - gi.a_base] = 1.0;
-    double c, lo, hi;
+)" << (any_direct ? "    if (gi.staged) sA[d_acol[col] - gi.a_base] = 1.0;\n    else gA[d_acol[col] - gi.a_base] = 1.0;\n"
+                  : "    sA[d_acol[col] - gi.a_base] = 1.0;\n")
+    << R"(    double c, lo, hi;
     if (col < NP) {
       c = pi[col]; lo = c; hi = c;
     } else {
@@ -500,12 +526,12 @@ assemble_kernel(const int B, const double* __restrict__ x, const double* __restr
   for (size_t t = 0; t < tmpl_text.size(); ++t)
     s << "      case " << t << ": stage_tmpl_" << t
       << "(xi + gi.xoff, pi, dir, lane, gi.first_col, d_tab + gi.atab_off, d_tab + gi.htab_off, d_tab + gi.ctab_off, "
-         "sA, sH, lbg, ubg, li, ui, qi, valid && pass == 0); break;\n";
+      << (tmpl_staged[t] ? "sA, sH" : "gA, gH") << ", lbg, ubg, li, ui, qi, valid && pass == 0); break;\n";
   s << R"(      default: break;
     }
   }
   __syncwarp();
-  if (valid) {
+  if ()" << (any_direct ? "valid && gi.staged" : "valid") << R"() {
     copy_out(av + static_cast<size_t>(inst) * lda + gi.a_base, sA, gi.a_len, lane);
     copy_out(hv + static_cast<size_t>(inst) * ldh + gi.h_base, sH, gi.h_len, lane);
   }

@@ -208,7 +208,8 @@ class OptimalControlProblem:
         return self.reference_
 
     def add_scalar_cost(self, cost) -> None:
-        _hcheck(host_lib().ocp_host_scripted_add_scalar_cost(self._h, SX._wrap(cost)._h))
+        cost = SX._wrap(cost)   # held until the call returns: a temporary's handle would be freed before it is read
+        _hcheck(host_lib().ocp_host_scripted_add_scalar_cost(self._h, cost._h))
 
     def add_vector_cost(self, weights: Sequence[float], cost: SX) -> None:
         w = _f64(weights)
