@@ -32,35 +32,10 @@
 
 #include "admm_common.cuh"
 #include "block_ring.cuh"
+#include "direct_layout.cuh"
 
 namespace ocpb200 {
 namespace direct {
-
-// Placement of the per-instance state:
-//   PLACE_MIXED  run-time mask (host plan: shared memory first, in ArrayId order; rest in a global slab)
-//   PLACE_SMEM   everything in shared memory, one CTA per SM (pointers are shared-space: LDS/STS)
-//   PLACE_MULTI  vectors, A values and small scratch in shared memory, factor blocks / index
-//                arrays / rarely used vectors in global memory (L2-resident): ~65 KB per CTA, so that
-//                three CTAs share an SM and hide each other's dependent-latency chains
-//   PLACE_BIG    one CTA per SM for problems whose factor does not fit: vectors, A values, scratch and
-//                index arrays in shared memory, factor blocks and set-up / check vectors in global memory
-enum Placement { PLACE_MIXED = 0, PLACE_SMEM = 1, PLACE_MULTI = 2, PLACE_BIG = 3 };
-
-// arrays of the per-instance state, in shared-memory priority order
-enum ArrayId {
-  AR_X = 0, AR_Q, AR_B, AR_Z, AR_Y, AR_L, AR_U, AR_CTYPE, AR_W, AR_AVAL, AR_SCRATCH, AR_STAGE, AR_IDX, AR_DINV, AR_LSUB,
-  AR_PVAL, AR_LP, AR_D, AR_E, AR_DX, AR_DY, AR_COUNT
-};
-// AR_STAGE: two pairs of block buffers in which the factorisation stages the blocks it multiplies
-// when the factor itself lives in the global slab; not allocated when everything is in shared memory.
-// throughput plan: vectors, A values, scratch, block staging buffers, index arrays + the small set-up /
-// scaling vectors in shared memory (109 KB for the quadrotor, two CTAs per SM); the factor blocks and
-// dx, dy (read at termination checks only) in the global slab
-__host__ __device__ constexpr bool multi_in_smem(int id) { return id <= AR_IDX || id == AR_PVAL || id == AR_D || id == AR_E; }
-__host__ __device__ constexpr bool big_in_smem(int id) { return id <= AR_IDX; }
-// latency plan: everything in shared memory except the block staging buffers (not needed) and dx, which only the
-// termination checks touch -- with it the H = 20 quadrotor is 1.7 KB over the 227 KB of an SM
-__host__ __device__ constexpr bool smem_in_smem(int id) { return id != AR_STAGE && id != AR_DX; }
 
 constexpr int kMaxRing = 8;   // ring slots per chain
 
@@ -85,34 +60,6 @@ struct Work {
   double *D, *E, *dx, *dy;
 };
 
-__host__ __device__ inline size_t array_doubles_nominal(const PatternDev& P, int id);
-__host__ __device__ inline size_t array_doubles(const PatternDev& P, int id) {
-  const size_t sz = array_doubles_nominal(P, id);
-  return sz > 0 ? ((sz + 1) & ~size_t(1)) + kCanaryDoubles : 0;   // guard doubles behind every array (0 unless OCP_B200_CANARY)
-}
-__host__ __device__ inline size_t array_doubles_nominal(const PatternDev& P, int id) {
-  const size_t n = P.n, m = P.m, bs = P.tri_bs, ld = P.tri_ld, nb = P.tri_nb, np = P.tri_np;
-  switch (id) {
-    case AR_X: case AR_Q: case AR_B: case AR_D: case AR_DX: return (n + 1) & ~size_t(1);
-    case AR_Z: case AR_Y: case AR_L: case AR_U: case AR_E: case AR_DY: return (m + 1) & ~size_t(1);
-#ifdef OCP_B200_CANARY_SELFTEST   // negative control of the guard check: the round-2 bug (w sized m, written up to n) on purpose
-    case AR_W: return (m + 1) & ~size_t(1);
-#else
-    case AR_W: return ((m > n ? m : n) + 1) & ~size_t(1);   // also the Ruiz scratch of the n column norms (QP-only handles may have m < n)
-#endif
-    case AR_CTYPE: return (m + 7) / 8;
-    case AR_AVAL: return (size_t(P.nnz_a) + 1) & ~size_t(1);
-    case AR_PVAL: return (size_t(P.nnz_p) + 1) & ~size_t(1);
-    case AR_DINV: case AR_LSUB: return nb * bs * ld;
-    case AR_IDX: return (size_t(P.idx_entries) * sizeof(idx_t) + 7) / 8;
-    case AR_STAGE: return size_t(P.stage_slots > 0 ? P.stage_slots : 4) * ((bs * ld + 1) & ~size_t(1));
-    case AR_LP: return (np * nb * bs + 1) & ~size_t(1);
-    case AR_SCRATCH: return 3 * np * (np + 1) + 2 * ((bs * ld + 1) & ~size_t(1)) + 2 * ((np * bs + 1) & ~size_t(1)) +
-                            ((np + 2) & ~size_t(1)) + 64;
-    default: return 0;
-  }
-}
-
 // With a compile-time placement (PLACE_SMEM / PLACE_MULTI) every pointer is derived from exactly
 // one base, so the compiler knows its address space and emits LDS/STS or LDG/STG, not generic LD.
 template <int kPlace>
@@ -120,8 +67,8 @@ __device__ __forceinline__ void carve(Work& W, const PatternDev& P, uint32_t sme
   double* ptr[AR_COUNT];
 #pragma unroll
   for (int id = 0; id < AR_COUNT; ++id) {
-    const size_t sz = (kPlace == PLACE_SMEM && id == AR_STAGE) ? 0 : ((array_doubles(P, id) + 1) & ~size_t(1));
-    const bool in_smem = kPlace == PLACE_SMEM ? smem_in_smem(id) || id == AR_STAGE : (kPlace == PLACE_MULTI ? multi_in_smem(id) : (kPlace == PLACE_BIG ? big_in_smem(id) : (smem_mask >> id & 1u) != 0));
+    const size_t sz = slot_doubles(P, kPlace, id);
+    const bool in_smem = ((kPlace == PLACE_MIXED ? smem_mask : placement_mask(kPlace)) >> id & 1u) != 0;
     if (in_smem) { ptr[id] = sm; sm += sz; }
     else { ptr[id] = gl; gl += sz; }
     if (kCanaryDoubles > 0 && sz > 0) {   // guard doubles at the end of the array's slot

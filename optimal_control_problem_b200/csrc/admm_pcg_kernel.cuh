@@ -40,6 +40,13 @@ struct Work {
 __host__ __device__ inline size_t work_doubles(const PatternDev& P) {
   return size_t(P.nnz_a) + P.nnz_p + 9 * size_t(P.n) + 10 * size_t(P.m) + P.minv_doubles + (P.m + 7) / 8;
 }
+// index entries the resident kernel stages in shared memory behind its state: the arrays of the stage(...) list in
+// admm_solve_kernel, each padded to 8 entries -- the two must list the same arrays
+__host__ __device__ inline size_t staged_idx_entries(const PatternDev& P) {
+  auto pad8 = [](size_t v) { return (v + 7) & ~size_t(7); };
+  return 2 * pad8(P.n + 1) + 3 * pad8(P.nnz_a) + pad8(P.m + 1) + pad8(P.nnz_p) + pad8(P.nblk + 1) + pad8(P.n) +
+         pad8(P.n_long) + pad8(P.n_short);
+}
 
 __device__ inline void carve(Work& W, double* base, const PatternDev& P) {
   double* p = base;
@@ -352,7 +359,7 @@ admm_solve_kernel(const PatternDev P, const ocp_b200_settings S, const SolveArgs
   if (kResident) {
     double* base = reinterpret_cast<double*>(smem_raw);
     carve(W, base, P);
-    // index structures move into shared memory once per CTA
+    // index structures move into shared memory once per CTA (staged_idx_entries sizes this list)
     idx_t* ip = reinterpret_cast<idx_t*>(base + work_doubles(P));
     auto stage = [&](const idx_t*& ptr, int count) {
       const idx_t* src = ptr;

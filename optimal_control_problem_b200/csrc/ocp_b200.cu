@@ -21,6 +21,7 @@
 #include "admm_pcg_kernel.cuh"
 #include "compact_launch.h"
 #include "direct_launch.h"
+#include "direct_layout.cuh"
 #include "ocp_b200_model.h"
 
 namespace ocpb200 {
@@ -102,8 +103,6 @@ struct DevBuf {
   void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 
-int pad8(int v) { return (v + 7) & ~7; }
-
 // rows with at least kLongRow entries are handled by four lanes each in the row-wise products, the others by one
 // thread.  Measured (quadrotor, rows of <= 17 entries): one thread per row beats four lanes per row by 7 %.
 constexpr int kLongRow = 64;
@@ -112,10 +111,13 @@ constexpr int kStageSlots = 8, kStageSlotsMin = 4;
 
 }  // namespace
 
+// One launch configuration of the ADMM solve.  place: -1 the PCG kernel, 0-3 the direct kernel under that
+// ocpb200::direct::Placement, 4 the compact kernel.
 struct LaunchPlan {
-  int place = 0, threads = 256, smem_bytes = 0, max_ctas = 1;
-  uint32_t smem_mask = 0;
-  size_t slab_doubles = 0;
+  int place = -1, threads = 0, smem_bytes = 0, max_ctas = 1;
+  uint32_t smem_mask = 0;    // direct kernel: which state arrays live in shared memory
+  int compact_flags = 0;     // compact kernel: which streamed vectors moved into shared memory
+  size_t slab_doubles = 0;   // per-CTA global slab
 };
 
 struct ocp_b200_solver {
@@ -134,18 +136,13 @@ struct ocp_b200_solver {
   DevBuf<uint32_t> d_arena;
   ocpb200::CompactIdx cidx{};
   int compact_ok = 0;
-  int compact_flags = 0;   // which streamed vectors moved into shared memory
   // stage library
   void* lib = nullptr;
   model_assemble_fn assemble = nullptr;
   model_objective_fn objective = nullptr;
   // launch configuration
-  int num_sms = 0, threads = 512, resident = 0, smem_bytes = 0, max_ctas = 0;
-  size_t slab_doubles = 0;
-  int use_direct = 0;          // 1: admm_direct_kernel (block-tridiagonal LDL'), 0: PCG kernel
-  int place = 0;               // direct kernel: ocpb200::direct::Placement of the throughput plan
-  LaunchPlan deep, wide;       // latency plan (1 CTA/SM) and throughput plan (2 CTAs/SM)
-  uint32_t smem_mask = 0;      // direct kernel: which state arrays live in shared memory
+  int num_sms = 0;
+  LaunchPlan deep, wide;       // latency plan (batches of at most one instance per SM) and throughput plan
   // workspaces (device)
   DevBuf<double> hv, q, av, l, u, solx, soly, info, slab, trace;
   DevBuf<double> x, p, frames, lbx, ubx, lbg, ubg, f, stats;
@@ -392,170 +389,115 @@ int upload_pattern(ocp_b200_solver* s, int num_blocks, const int* block_ptr) {
 }
 
 // Chooses the kernel for the current settings and lays out its per-instance state: shared
-// memory first, in the priority order of direct::ArrayId, the rest in a per-CTA global slab.
+// memory first, the rest in a per-CTA global slab.
 int plan_launch(ocp_b200_solver* s) {
   const PatternDev& P = s->pat;
   int max_optin = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, s->device));
-  s->use_direct = (s->settings.pcg_precond == OCP_B200_PRECOND_BLOCK_TRIDIAG && P.tri_ok) ? 1 : 0;
-  int per_sm = 1;
-  if (s->use_direct) {
-    namespace D = ocpb200::direct;
-    const int count = D::plan_array_count();
-    // Two plans are kept.  `wide`: 2 CTAs per SM (vectors, A values, index arrays and scratch in
-    // shared memory, factor blocks in an L2-resident slab) -- the throughput plan, used when the
-    // batch has more instances than SMs.  `deep`: 1 CTA per SM with as much state as fits in shared
-    // memory (everything, for the H=20 quadrotor) -- the latency plan, used for small batches.
-    // OCP_B200_PLAN = smem | multi | mixed forces one of them (diagnostics).
-    const char* env = std::getenv("OCP_B200_PLAN");
-    size_t multi_smem = 0, multi_slab = 0, big_smem = 0, big_slab = 0, all = 0;
-    const int stage_id = D::plan_stage_array();   // not allocated by the all-shared-memory plan
-    auto measure = [&]() {
-      multi_smem = multi_slab = big_smem = big_slab = all = 0;
-      for (int id = 0; id < count; ++id) {
-        const size_t sz = (D::plan_array_doubles(P, id) + 1) & ~size_t(1);
-        if (D::plan_smem_in_smem(id)) all += sz;
-        (D::plan_multi_in_smem(id) ? multi_smem : multi_slab) += sz;
-        (D::plan_big_in_smem(id) ? big_smem : big_slab) += sz;
-      }
-    };
-    s->pat.stage_slots = kStageSlotsMin;
-    measure();
-    auto make_plan = [&](int place, LaunchPlan& L) -> int {
-      D::KernelInfo kx{};
-      const D::EntryPoints& ep = D::entry_points(place);
-      CUDA_TRY(ep.kernel_info(&kx));
-      L.place = place;
-      L.threads = kx.threads;
-      CUDA_TRY(ep.set_max_dynamic_smem(max_optin - kx.static_smem));
-      if (place == 2) {
-        L.smem_mask = 0;
-        L.smem_bytes = static_cast<int>(multi_smem * sizeof(double));
-        L.slab_doubles = (multi_slab + 15) & ~size_t(15);
-      } else if (place == 3) {
-        L.smem_mask = 0;
-        L.smem_bytes = static_cast<int>(big_smem * sizeof(double));
-        L.slab_doubles = (big_slab + 15) & ~size_t(15);
-      } else {
-        size_t avail = (size_t(max_optin) - kx.static_smem) / sizeof(double), used = 0, slab = 0;
-        uint32_t mask = 0;
-        // mixed placement: shared memory goes first to what is accessed at random or sits on the
-        // sequential path (solve vector, x, w, the block ring, the border scratch); vectors that are
-        // only streamed row by row (z, y, l, u) and the matrices follow while space lasts
-        std::vector<int> order;
-        if (place == 1) {
-          for (int id = 0; id < count; ++id) order.push_back(id);
-        } else {
-          D::plan_mixed_priority(order);
-        }
-        // OCP_B200_FORCE_STREAM keeps the factor in the global slab even when it would fit (tests of the
-        // streamed solve on small problems)
-        const bool force_stream = place == 0 && std::getenv("OCP_B200_FORCE_STREAM") != nullptr;
-        for (int id : order) {
-          const size_t sz = (place == 1 && id == stage_id) ? 0 : ((D::plan_array_doubles(P, id) + 1) & ~size_t(1));
-          const bool keep_out = (force_stream && D::plan_is_factor_array(id)) || (place == 1 && !D::plan_smem_in_smem(id));
-          if (!keep_out && (place == 1 || used + sz <= avail)) { mask |= 1u << id; used += sz; }
-          else slab += sz;
-        }
-        L.smem_mask = mask;
-        L.smem_bytes = static_cast<int>(used * sizeof(double));
-        L.slab_doubles = (slab + 15) & ~size_t(15);
-      }
-      int occ = 1;
-      CUDA_TRY(ep.occupancy(L.smem_bytes, &occ));
-      L.max_ctas = std::max(1, occ) * s->num_sms;
-      return OCP_B200_OK;
-    };
-    D::KernelInfo ki{}, km{};
-    CUDA_TRY(D::kSmem.kernel_info(&ki));
-    CUDA_TRY(D::kMulti.kernel_info(&km));
-    const bool fits_all = all * sizeof(double) + ki.static_smem <= size_t(max_optin);
-    const bool fits_multi = (multi_smem * sizeof(double) + km.static_smem + 1024) * 2 <= size_t(228) * 1024;
-    D::KernelInfo kb{};
-    CUDA_TRY(D::kBig.kernel_info(&kb));
-    bool fits_big = big_smem * sizeof(double) + kb.static_smem <= size_t(max_optin);
-    const bool forced_big = env && !std::strcmp(env, "big");
-    if (fits_big && ((!fits_all && !fits_multi) || forced_big)) {
-      // the 1-CTA/SM slab plan is the only one: widen the staging area to a ring of 4 blocks per
-      // sweep chain (asynchronous bulk copies, tri_twisted.cuh) when shared memory allows
-      s->pat.stage_slots = kStageSlots;
-      measure();
-      if (big_smem * sizeof(double) + kb.static_smem > size_t(max_optin)) { s->pat.stage_slots = kStageSlotsMin; measure(); }
-    }
-    int deep = fits_all ? 1 : (fits_big ? 3 : 0), wide = fits_multi ? 2 : deep;
-    if (env && !std::strcmp(env, "multi") && fits_multi) deep = wide = 2;
-    else if (env && !std::strcmp(env, "mixed")) deep = wide = 0;
-    else if (env && !std::strcmp(env, "smem") && fits_all) deep = wide = 1;
-    else if (env && !std::strcmp(env, "big") && fits_big) deep = wide = 3;
-    RC_TRY(make_plan(deep, s->deep));
-    RC_TRY(make_plan(wide, s->wide));
-    // compact throughput plan (admm_compact_kernel.cuh): index templates, streamed slab vectors, four CTAs per SM --
-    // taken when it keeps more threads resident than the plan above (OCP_B200_PLAN=compact forces it, any other value
-    // of OCP_B200_PLAN keeps it out).  q, then l and u, move from the slab into shared memory while the residency
-    // target still holds.
-    s->compact_flags = 0;
-    if (s->compact_ok && (P.tri_bs == 16 || P.tri_bs == 20) && P.tri_ld == P.tri_bs + 2 && (!env || !std::strcmp(env, "compact"))) {
-      namespace K = ocpb200::compact;
-      D::KernelInfo kc{};
-      CUDA_TRY(K::kernel_info(P.tri_bs, &kc));
-      CUDA_TRY(K::set_max_dynamic_smem(P.tri_bs, max_optin - kc.static_smem));
-      int best_flags = -1, best_occ = 0;
-      size_t best_sm = 0, best_sl = 0;
-      for (int flags : {3, 1, 0}) {   // most shared memory first
-        size_t sm_d = 0, sl_d = 0;
-        bool lay_ok = false;
-        K::plan_sizes(P, s->cidx.arena_words, flags, &sm_d, &sl_d, &lay_ok);
-        if (!lay_ok || sm_d * sizeof(double) + kc.static_smem > size_t(max_optin)) continue;
-        // residency by hand: the occupancy calculator answers 1 for a kernel that allocates Tensor Memory (it cannot know
-        // how many of the 512 columns a CTA will ask for); the compact kernel takes 128 of them when BS == 16
-        int occ = 0;
-        {
-          int smem_sm = 0, regs_sm = 0;
-          CUDA_TRY(cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, s->device));
-          CUDA_TRY(cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, s->device));
-          const int regs_cta = ((kc.regs + 7) / 8 * 8) * kc.threads;
-          const size_t smem_cta = sm_d * sizeof(double) + kc.static_smem + 1024;   // 1 KB reserved per CTA
-          occ = std::min({regs_sm / std::max(1, regs_cta), static_cast<int>(size_t(smem_sm) / smem_cta), 2048 / kc.threads,
-                          P.tri_bs == 16 ? 512 / 128 : 32});
-        }
-        if (occ > best_occ && best_occ < K::kCtasPerSm) { best_occ = occ; best_flags = flags; best_sm = sm_d; best_sl = sl_d; }
-      }
-      if (best_flags >= 0) {
-        const int occ = std::min(best_occ, K::kCtasPerSm);
-        if (occ * kc.threads > (s->wide.max_ctas / s->num_sms) * s->wide.threads || env) {
-          s->wide.place = 4; s->wide.threads = kc.threads; s->wide.smem_bytes = static_cast<int>(best_sm * sizeof(double));
-          s->wide.smem_mask = 0; s->wide.slab_doubles = best_sl; s->wide.max_ctas = occ * s->num_sms;
-          s->compact_flags = best_flags;
-          if (env) s->deep = s->wide;
-        }
-      }
-    }
-    s->place = s->wide.place; s->threads = s->wide.threads; s->smem_bytes = s->wide.smem_bytes;
-    s->smem_mask = s->wide.smem_mask; s->slab_doubles = s->wide.slab_doubles;
-    s->resident = s->deep.place == 1 ? 1 : 0;
-    per_sm = s->wide.max_ctas / s->num_sms;
-  } else {
-    s->threads = 512;
-    const size_t idx_entries = size_t(pad8(P.n + 1)) * 2 + size_t(pad8(P.nnz_a)) * 3 + pad8(P.m + 1) + pad8(P.nnz_p) +
-                               pad8(P.nblk + 1) + pad8(P.n) + pad8(P.n_long) + pad8(P.n_short);
-    const size_t want = ocpb200::pcg::work_doubles(P) * sizeof(double) + idx_entries * sizeof(idx_t);
+  if (s->settings.pcg_precond != OCP_B200_PRECOND_BLOCK_TRIDIAG || !P.tri_ok) {
+    // PCG kernel, one plan for every batch size: its state in shared memory when it fits ("resident"), else in the slab
+    LaunchPlan L;
+    L.threads = 512;
+    const size_t want = ocpb200::pcg::work_doubles(P) * sizeof(double) + ocpb200::pcg::staged_idx_entries(P) * sizeof(idx_t);
     cudaFuncAttributes fa{};
     CUDA_TRY(cudaFuncGetAttributes(&fa, ocpb200::pcg::admm_solve_kernel<true>));
-    const size_t avail = size_t(max_optin) - fa.sharedSizeBytes;
-    s->resident = want <= avail ? 1 : 0;
-    s->smem_bytes = s->resident ? static_cast<int>(want) : 0;
-    if (s->resident)
+    int per_sm = 1;
+    if (want <= size_t(max_optin) - fa.sharedSizeBytes) {
+      L.smem_bytes = static_cast<int>(want);
       CUDA_TRY(cudaFuncSetAttribute(ocpb200::pcg::admm_solve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     max_optin - static_cast<int>(fa.sharedSizeBytes)));
-    s->slab_doubles = (ocpb200::pcg::work_doubles(P) + 15) & ~size_t(15);
-    if (s->resident)
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ocpb200::pcg::admm_solve_kernel<true>,
-                                                             s->threads, s->smem_bytes));
-    else
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ocpb200::pcg::admm_solve_kernel<false>,
-                                                             s->threads, 0));
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ocpb200::pcg::admm_solve_kernel<true>, L.threads,
+                                                             L.smem_bytes));
+    } else {
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ocpb200::pcg::admm_solve_kernel<false>, L.threads, 0));
+    }
+    // reported for the resident kernel as well, although it launches without a slab
+    L.slab_doubles = (ocpb200::pcg::work_doubles(P) + 15) & ~size_t(15);
+    L.max_ctas = std::max(1, per_sm) * s->num_sms;
+    s->deep = s->wide = L;
+    return OCP_B200_OK;
   }
-  s->max_ctas = std::max(1, per_sm) * s->num_sms;
+  namespace D = ocpb200::direct;
+  // Two plans are kept.  `wide`: 2 CTAs per SM (vectors, A values, index arrays and scratch in
+  // shared memory, factor blocks in an L2-resident slab) -- the throughput plan, used when the
+  // batch has more instances than SMs.  `deep`: 1 CTA per SM with as much state as fits in shared
+  // memory (everything, for the H=20 quadrotor) -- the latency plan, used for small batches.
+  // OCP_B200_PLAN = smem | multi | mixed forces one of them (diagnostics).
+  const char* env = std::getenv("OCP_B200_PLAN");
+  const bool force_stream = std::getenv("OCP_B200_FORCE_STREAM") != nullptr;
+  auto smem_bytes = [&](int place) { return D::plan_state(P, place, 0, false).smem_doubles * sizeof(double); };
+  s->pat.stage_slots = kStageSlotsMin;
+  auto make_plan = [&](int place, LaunchPlan& L) -> int {
+    D::KernelInfo kx{};
+    const D::EntryPoints& ep = D::entry_points(place);
+    CUDA_TRY(ep.kernel_info(&kx));
+    CUDA_TRY(ep.set_max_dynamic_smem(max_optin - kx.static_smem));
+    const D::StateLayout st = D::plan_state(P, place, (size_t(max_optin) - kx.static_smem) / sizeof(double), force_stream);
+    const int bytes = static_cast<int>(st.smem_doubles * sizeof(double));
+    int occ = 1;
+    CUDA_TRY(ep.occupancy(bytes, &occ));
+    L = LaunchPlan{place, kx.threads, bytes, std::max(1, occ) * s->num_sms, st.mask, 0, st.slab_doubles};
+    return OCP_B200_OK;
+  };
+  D::KernelInfo ki{}, km{}, kb{};
+  CUDA_TRY(D::kSmem.kernel_info(&ki));
+  CUDA_TRY(D::kMulti.kernel_info(&km));
+  CUDA_TRY(D::kBig.kernel_info(&kb));
+  const bool fits_all = smem_bytes(D::PLACE_SMEM) + ki.static_smem <= size_t(max_optin);
+  const bool fits_multi = (smem_bytes(D::PLACE_MULTI) + km.static_smem + 1024) * 2 <= size_t(228) * 1024;
+  const bool fits_big = smem_bytes(D::PLACE_BIG) + kb.static_smem <= size_t(max_optin);
+  const bool forced_big = env && !std::strcmp(env, "big");
+  if (fits_big && ((!fits_all && !fits_multi) || forced_big)) {
+    // the 1-CTA/SM slab plan is the only one: widen the staging area to a ring of 4 blocks per
+    // sweep chain (asynchronous bulk copies, tri_twisted.cuh) when shared memory allows
+    s->pat.stage_slots = kStageSlots;
+    if (smem_bytes(D::PLACE_BIG) + kb.static_smem > size_t(max_optin)) s->pat.stage_slots = kStageSlotsMin;
+  }
+  int deep = fits_all ? 1 : (fits_big ? 3 : 0), wide = fits_multi ? 2 : deep;
+  if (env && !std::strcmp(env, "multi") && fits_multi) deep = wide = 2;
+  else if (env && !std::strcmp(env, "mixed")) deep = wide = 0;
+  else if (env && !std::strcmp(env, "smem") && fits_all) deep = wide = 1;
+  else if (env && !std::strcmp(env, "big") && fits_big) deep = wide = 3;
+  RC_TRY(make_plan(deep, s->deep));
+  RC_TRY(make_plan(wide, s->wide));
+  // compact throughput plan (admm_compact_kernel.cuh): index templates, streamed slab vectors, four CTAs per SM --
+  // taken when it keeps more threads resident than the plan above (OCP_B200_PLAN=compact forces it, any other value
+  // of OCP_B200_PLAN keeps it out).  q, then l and u, move from the slab into shared memory while the residency
+  // target still holds.
+  if (s->compact_ok && (P.tri_bs == 16 || P.tri_bs == 20) && P.tri_ld == P.tri_bs + 2 && (!env || !std::strcmp(env, "compact"))) {
+    namespace K = ocpb200::compact;
+    D::KernelInfo kc{};
+    CUDA_TRY(K::kernel_info(P.tri_bs, &kc));
+    CUDA_TRY(K::set_max_dynamic_smem(P.tri_bs, max_optin - kc.static_smem));
+    int best_flags = -1, best_occ = 0;
+    size_t best_sm = 0, best_sl = 0;
+    for (int flags : {3, 1, 0}) {   // most shared memory first
+      size_t sm_d = 0, sl_d = 0;
+      bool lay_ok = false;
+      K::plan_sizes(P, s->cidx.arena_words, flags, &sm_d, &sl_d, &lay_ok);
+      if (!lay_ok || sm_d * sizeof(double) + kc.static_smem > size_t(max_optin)) continue;
+      // residency by hand: the occupancy calculator answers 1 for a kernel that allocates Tensor Memory (it cannot know
+      // how many of the 512 columns a CTA will ask for); the compact kernel takes 128 of them when BS == 16
+      int occ = 0;
+      {
+        int smem_sm = 0, regs_sm = 0;
+        CUDA_TRY(cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, s->device));
+        CUDA_TRY(cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, s->device));
+        const int regs_cta = ((kc.regs + 7) / 8 * 8) * kc.threads;
+        const size_t smem_cta = sm_d * sizeof(double) + kc.static_smem + 1024;   // 1 KB reserved per CTA
+        occ = std::min({regs_sm / std::max(1, regs_cta), static_cast<int>(size_t(smem_sm) / smem_cta), 2048 / kc.threads,
+                        P.tri_bs == 16 ? 512 / 128 : 32});
+      }
+      if (occ > best_occ && best_occ < K::kCtasPerSm) { best_occ = occ; best_flags = flags; best_sm = sm_d; best_sl = sl_d; }
+    }
+    if (best_flags >= 0) {
+      const int occ = std::min(best_occ, K::kCtasPerSm);
+      if (occ * kc.threads > (s->wide.max_ctas / s->num_sms) * s->wide.threads || env) {
+        s->wide = LaunchPlan{4, kc.threads, static_cast<int>(best_sm * sizeof(double)), occ * s->num_sms, 0, best_flags, best_sl};
+        if (env) s->deep = s->wide;
+      }
+    }
+  }
   return OCP_B200_OK;
 }
 
@@ -630,32 +572,26 @@ int launch_admm(ocp_b200_solver* s, SolveArgs& A, cudaStream_t st) {
   CUDA_TRY(cudaMemsetAsync(s->counter.p, 0, sizeof(int), st));
   A.counter = s->counter.p;
   A.phase = s->profiling >= 2 ? s->phase.p : nullptr;
-  int grid = std::min(A.B, s->max_ctas);
+  // small batches (at most one instance per SM): the latency plan; otherwise the throughput plan
+  const LaunchPlan& L = A.B <= s->num_sms ? s->deep : s->wide;
+  const int grid = std::min(A.B, L.max_ctas);
   ProfScope prof(s, OCP_B200_PROF_ADMM, st);
-  if (s->use_direct) {
-    // small batches (at most one instance per SM): the latency plan; otherwise the throughput plan
-    const LaunchPlan& L = A.B <= s->num_sms ? s->deep : s->wide;
-    grid = std::min(A.B, L.max_ctas);
-    A.slab = nullptr; A.slab_doubles = L.slab_doubles;
-    if (L.slab_doubles > 0) {
-      CUDA_TRY(s->slab.reserve(size_t(grid) * L.slab_doubles));
-      A.slab = s->slab.p;
-    }
-    if (L.place == 4)
-      CUDA_TRY(ocpb200::compact::launch(s->pat.tri_bs, grid, L.smem_bytes, st, s->pat, s->cidx, s->settings, A, s->compact_flags));
-    else
-      CUDA_TRY(ocpb200::direct::entry_points(L.place).launch(grid, L.smem_bytes, st, s->pat, s->settings, A, L.smem_mask));
-  } else if (s->resident) {
-    A.slab = nullptr; A.slab_doubles = 0;
+  // the resident PCG kernel (state in shared memory) takes no slab
+  const bool slab = L.slab_doubles > 0 && (L.place >= 0 || L.smem_bytes == 0);
+  A.slab = nullptr; A.slab_doubles = slab ? L.slab_doubles : 0;
+  if (slab) {
+    CUDA_TRY(s->slab.reserve(size_t(grid) * L.slab_doubles));
+    A.slab = s->slab.p;
+  }
+  if (L.place < 0) {
     ocp_b200_settings t = s->settings;
     if (t.pcg_precond == OCP_B200_PRECOND_BLOCK_TRIDIAG) t.pcg_precond = OCP_B200_PRECOND_BLOCK_JACOBI;
-    ocpb200::pcg::admm_solve_kernel<true><<<grid, s->threads, s->smem_bytes, st>>>(s->pat, t, A);
+    if (L.smem_bytes > 0) ocpb200::pcg::admm_solve_kernel<true><<<grid, L.threads, L.smem_bytes, st>>>(s->pat, t, A);
+    else ocpb200::pcg::admm_solve_kernel<false><<<grid, L.threads, 0, st>>>(s->pat, t, A);
+  } else if (L.place == 4) {
+    CUDA_TRY(ocpb200::compact::launch(s->pat.tri_bs, grid, L.smem_bytes, st, s->pat, s->cidx, s->settings, A, L.compact_flags));
   } else {
-    CUDA_TRY(s->slab.reserve(size_t(grid) * s->slab_doubles));
-    A.slab = s->slab.p; A.slab_doubles = s->slab_doubles;
-    ocp_b200_settings t = s->settings;
-    if (t.pcg_precond == OCP_B200_PRECOND_BLOCK_TRIDIAG) t.pcg_precond = OCP_B200_PRECOND_BLOCK_JACOBI;
-    ocpb200::pcg::admm_solve_kernel<false><<<grid, s->threads, 0, st>>>(s->pat, t, A);
+    CUDA_TRY(ocpb200::direct::entry_points(L.place).launch(grid, L.smem_bytes, st, s->pat, s->settings, A, L.smem_mask));
   }
   CUDA_TRY(cudaGetLastError());
   s->launches++;
@@ -1033,8 +969,11 @@ int ocp_b200_get_dims(const ocp_b200_solver* s, int* n, int* m, int* nnz_h, int*
   if (m) *m = s->m;
   if (nnz_h) *nnz_h = s->nnz_h;
   if (nnz_a) *nnz_a = s->nnz_a;
-  if (smem_bytes) *smem_bytes = s->smem_bytes;
-  if (resident) *resident = s->resident | (s->use_direct << 1) | (s->place << 2);
+  if (smem_bytes) *smem_bytes = s->wide.smem_bytes;
+  // PCG kernel: bit 0 = its state is in shared memory.  Direct kernels: bit 0 = the latency plan keeps everything in
+  // shared memory, bit 1 set, bits 2 and up = placement of the throughput plan.
+  if (resident)
+    *resident = s->wide.place < 0 ? s->wide.smem_bytes > 0 : (s->deep.place == 1) | 2 | s->wide.place << 2;
   return OCP_B200_OK;
 }
 
@@ -1143,20 +1082,12 @@ int ocp_b200_get_plan(const ocp_b200_solver* s, int* v, int count) {
   if (!s || !v || count < 0) return fail(OCP_B200_ERR_INVALID, "solver/v is NULL");
   int o[OCP_B200_PLAN_COUNT] = {0};
   const int sms = std::max(1, s->num_sms);
-  if (s->use_direct) {
-    const LaunchPlan* L[2] = {&s->wide, &s->deep};
-    for (int k = 0; k < 2; ++k) {
-      o[5 * k + 0] = L[k]->place; o[5 * k + 1] = L[k]->threads; o[5 * k + 2] = L[k]->smem_bytes;
-      o[5 * k + 3] = L[k]->max_ctas / sms; o[5 * k + 4] = static_cast<int>(L[k]->slab_doubles * sizeof(double) / 1024);
-    }
-  } else {
-    o[OCP_B200_PLAN_WIDE_PLACE] = o[OCP_B200_PLAN_DEEP_PLACE] = -1;
-    o[OCP_B200_PLAN_WIDE_THREADS] = o[OCP_B200_PLAN_DEEP_THREADS] = s->threads;
-    o[OCP_B200_PLAN_WIDE_SMEM] = o[OCP_B200_PLAN_DEEP_SMEM] = s->smem_bytes;
-    o[OCP_B200_PLAN_WIDE_CTAS_SM] = o[OCP_B200_PLAN_DEEP_CTAS_SM] = s->max_ctas / sms;
-    o[OCP_B200_PLAN_WIDE_SLAB_KB] = o[OCP_B200_PLAN_DEEP_SLAB_KB] = static_cast<int>(s->slab_doubles * sizeof(double) / 1024);
+  const LaunchPlan* L[2] = {&s->wide, &s->deep};
+  for (int k = 0; k < 2; ++k) {
+    o[5 * k + 0] = L[k]->place; o[5 * k + 1] = L[k]->threads; o[5 * k + 2] = L[k]->smem_bytes;
+    o[5 * k + 3] = L[k]->max_ctas / sms; o[5 * k + 4] = static_cast<int>(L[k]->slab_doubles * sizeof(double) / 1024);
   }
-  o[OCP_B200_PLAN_TRI_OK] = s->use_direct;
+  o[OCP_B200_PLAN_TRI_OK] = s->wide.place >= 0;
   o[OCP_B200_PLAN_TRI_NP] = s->pat.tri_np; o[OCP_B200_PLAN_TRI_BS] = s->pat.tri_bs; o[OCP_B200_PLAN_TRI_NB] = s->pat.tri_nb;
   o[OCP_B200_PLAN_NNZ_P] = s->nnz_p;
   o[OCP_B200_PLAN_NUM_SMS] = s->num_sms;
